@@ -1,6 +1,6 @@
 """Benchmark of the Seg2Eye SPADE+Style G+D training step (BASELINE.json metric: G+D train images/s).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--res R1|R2] [--batch B]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--res R1|R2] [--batch B] [--dump-outputs DIR]
 
 One "step" = one Pix2PixTrainer.run_generator_one_step + run_discriminator_one_step over one synthetic batch
 (labels: eye-shaped 4-class ellipses; images/targets U(-1,1); reference-initialised weights).  Prints ONE JSON line.
@@ -12,6 +12,11 @@ One "step" = one Pix2PixTrainer.run_generator_one_step + run_discriminator_one_s
              CUDA-event durations inside the timed region, against the measured bf16 GEMM peak.
 `cpu_baseline` / --impl reference: the oracle port (plain fp32 PyTorch restatement of the reference, the reference
              itself is Python and does not travel to the GPU box) timed on the host cores on a bounded sample.
+--dump-outputs DIR: writes what one step of the timed path returns to a caller as DIR/<name>.npy (float32): the generated
+             image and the losses of a training step, the integer images of a c4 sweep.  A training step is dumped from
+             the seeded initial weights: after the timed steps they are restored, with a fresh optimizer, and the timed
+             path (the same CUDA graphs, the same batch) runs one more step.  Inputs and weights are seeded, so two builds
+             of the project run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -96,6 +101,22 @@ def workload_config(res, batch, world, workload="c2"):
                                 "c5": "BASELINE.json configs[4]"}[workload],
             "global_batch": batch * world, "parallelism": "dp%d" % world,
             "l2_policy": "inputs+activations per step (>1 GB) exceed the 126 MB L2"}
+
+
+DUMP_SAMPLE = 1 << 22   # an output with more elements is dumped as a fixed sample of this many (16 MB in float32)
+
+
+def dump_outputs(out_dir, arrays):
+    """<out_dir>/<name>.npy in float32 for each array; a larger one than DUMP_SAMPLE elements is replaced by the same
+    seeded sample of its flattened elements (in index order) on every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name.replace("/", "_") + ".npy"), a.numpy())
 
 
 def load_peaks():
@@ -288,6 +309,8 @@ def run_ours(args):
     with contextlib.redirect_stdout(io.StringIO()):
         tr = Pix2PixTrainer(opt)
     m = tr.pix2pix_model
+    nets = [net for net in (m.netG, m.netD, m.netE) if net is not None]
+    seeded = [{k: v.clone() for k, v in net.state_dict().items()} for net in nets] if args.dump_outputs else None
     host = O.synth_batch(oopt, args.batch, 1234 + rank)
     if m.netE is None:
         host.pop("style_image")
@@ -316,8 +339,7 @@ def run_ours(args):
     for _ in range(2):
         step(dev)
     launches_per_step = (L.launches - n0) // 2
-    prof = ops.profile_end(os.path.join(REPO, 'gpurun_out', 'kernel_profile_%s_%s_b%d.tsv' % (args.workload, args.res, args.batch))
-                           if (rank == 0 and os.path.isdir(os.path.join(REPO, 'gpurun_out'))) else None)
+    prof = ops.profile_end()
     barrier()
     if args.ncu_step:   # one eager step delimited by cudaProfilerStart/Stop (ncu --profile-from-start off)
         torch.cuda.synchronize()
@@ -363,6 +385,20 @@ def run_ours(args):
     ms_e2e = f0.elapsed_time(f1)
     sampler.stop_flag = True
     sampler.join(2)
+    if args.dump_outputs:
+        # The weight-gradient and loss reductions add with float atomics, so a step is reproducible to rounding only, and
+        # Adam(beta1 = 0) steps from the small initial weights amplify that: two seeded runs differ by 4e-3 in the image
+        # after two steps and are unrelated after five (tools/trajectory_repro.py, profiles/r03_trajectory_repro.txt).  The
+        # dumped step is therefore one more step of the timed path from the seeded weights and fresh optimizers, loaded the
+        # way a checkpoint is (the graphs re-pack the bf16 weights themselves before the replay).
+        for net, sd in zip(nets, seeded):
+            net.load_state_dict(sd)
+        tr.reset_optimizers()
+        step(dev)
+        barrier()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"generated": tr.get_latest_generated(),
+                                             **{"loss_" + k: v for k, v in tr.get_latest_losses().items()}})
 
     t = torch.tensor([ms, ms_e2e], device="cuda", dtype=torch.float64)
     if world > 1:
@@ -467,8 +503,7 @@ def run_c4(args):
     n0 = L.launches
     sweep(dev, True)
     launches = L.launches - n0
-    prof = ops.profile_end(os.path.join(REPO, "gpurun_out", "kernel_profile_c4_%s_b%d.tsv" % (args.res, nb))
-                           if os.path.isdir(os.path.join(REPO, "gpurun_out")) else None)
+    prof = ops.profile_end()
     sampler = ClockSampler(local)
     sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -490,6 +525,8 @@ def run_c4(args):
     ms_e2e = f0.elapsed_time(f1)
     sampler.stop_flag = True
     sampler.join(2)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"images": out_host})
     peaks = load_peaks()
     conv_ms, conv_tf = prof["tc_ms"], prof["tc_flop"] / 1e12
     achieved = conv_tf / (conv_ms / 1e3) if conv_ms > 0 else 0.0
@@ -541,7 +578,11 @@ def main():
     ap.add_argument("--mode", default="graph", choices=("graph", "eager"))
     ap.add_argument("--ncu-step", action="store_true", help="bracket one eager step with cudaProfilerStart/Stop")
     ap.add_argument("--precision", default="bf16", choices=("bf16", "tf32"), help="--impl library only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of one step of the timed path, from the seeded "
+                    "weights, to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     if args.res is None:
         args.res = {"c2": "R2", "c4": "R1", "c5": "S256"}[args.workload]
@@ -551,7 +592,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps, warmup = max(1, min(args.steps, 3)), min(args.warmup, 1)
+        steps, warmup = args.steps, args.warmup
         r = cpu_reference(args.res, steps, warmup, workload=args.workload)
         cb = {"value": r["value"], "unit": "images/s", "cores": r["cores"], "kind": "port",
               "sample": r["sample"] + " (oracle/seg2eye_oracle.py: fp32 PyTorch-CPU restatement of the reference; the reference "
@@ -570,7 +611,7 @@ def main():
         if rank != 0:
             return
         torch.cuda.set_device(int(os.environ.get("LOCAL_RANK", "0")))
-        r = library_reference(args.res, max(1, min(args.steps, 5)), max(1, min(args.warmup, 3)), args.batch, args.precision, args.workload)
+        r = library_reference(args.res, args.steps, args.warmup, args.batch, args.precision, args.workload)
         print(json.dumps({
             "impl": "library", "metric": "G+D train images/sec", "value": r["value"], "unit": "images/s", "n_gpus": 1,
             "ms_per_step": r["ms_per_step"], "higher_is_better": True, "dtype": args.precision, "data": "synthetic",

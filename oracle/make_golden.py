@@ -25,6 +25,7 @@ from oracle import seg2eye_oracle as O  # noqa: E402
 
 SMALL = dict(ngf=16, ndf=16, lambda_l1=10.0)   # 320x256, label_nc 4, w_dim 16, input_ns 4
 SEEDS = dict(G=101, D=202, E=303, batch=404)
+IMAGE_SUB = 16384   # samples kept of a generated 2x1x320x256 image
 
 
 def import_reference():
@@ -143,7 +144,8 @@ def main():
         fake = model.netG(seg, w)
         for h in hooks:
             h.remove()
-        g["G_fake"] = fake.numpy()
+        # images: a 1-in-10 subsample + norm / mean, which keeps the file small enough to commit
+        g["G_fake_sub"], g["G_fake_stat"] = sub(fake, IMAGE_SUB)
         for name, t in taps.items():
             g["G_tap_%s_sub" % name], g["G_tap_%s_stat" % name] = sub(t)
         sdg = model.netG.state_dict()
@@ -173,7 +175,11 @@ def main():
         trainer.run_discriminator_one_step(data)
         for k, v in trainer.get_latest_losses().items():
             g["step%d_loss_%s" % (it, k)] = v.detach().reshape(-1).numpy().astype(np.float64)
-        g["step%d_generated" % it] = trainer.get_latest_generated().detach().numpy()
+        gen = trainer.get_latest_generated().detach()
+        if it == 0:     # the first iteration generates from the same weights and inputs as the forward above: G_fake_*
+            assert torch.equal(gen, fake)
+        else:
+            g["step%d_generated_sub" % it], g["step%d_generated_stat" % it] = sub(gen, IMAGE_SUB)
     m = trainer.pix2pix_model
     post = dict(G=m.netG.state_dict(), D=m.netD.state_dict(), E=m.netE.state_dict())
     for net, keys in dict(

@@ -124,13 +124,7 @@ class Pix2PixTrainer():
                 self._eager_step('G', dict(self._static))
                 self._eager_step('D', dict(self._static))
                 if fresh:
-                    for o in opts:
-                        for st in o.state.values():
-                            st['exp_avg'].zero_()
-                            st['exp_avg_sq'].zero_()
-                        for g in o.param_groups:
-                            if g.get('_s2e_state') is not None:
-                                g['_s2e_state'][0].zero_()
+                    self.reset_optimizers()
                 for t, s0 in zip(tensors, snap0):
                     t.detach().copy_(s0)
             if multi:
@@ -189,6 +183,17 @@ class Pix2PixTrainer():
         ops.bump_weights_epoch()
         ops.repack_stale()   # the graphs re-pack after their own Adam; the restored weights need it once, here
         self._graphs = True
+
+    def reset_optimizers(self):
+        """Both optimizers as freshly constructed: zero Adam moments and step counts, written in place so that captured
+        CUDA graphs keep reading the same tensors."""
+        for o in (self.optimizer_G, self.optimizer_D):
+            for st in o.state.values():
+                st['exp_avg'].zero_()
+                st['exp_avg_sq'].zero_()
+            for g in o.param_groups:
+                if g.get('_s2e_state') is not None:
+                    g['_s2e_state'][0].zero_()
 
     def disable_cuda_graphs(self):
         self._graphs = False

@@ -101,7 +101,9 @@ def test_trainer_lr_schedule_and_errors():
     assert abs(tr.old_lr - (opt.lr - opt.lr / 7)) < 1e-12
     assert abs(tr.optimizer_D.param_groups[0]["lr"] - 2 * tr.old_lr) < 1e-12
     with pytest.raises(ValueError):
-        tr.pix2pix_model({"label": torch.zeros(1, 1, 8, 8), "style_image": torch.zeros(1, 4, 1, 8, 8)}, mode="bogus") \
+        # the inputs are pre-processed by our kernels on the model's device before the mode is looked at: on a machine with
+        # a GPU the model built with gpu_ids = [] moves there first
+        tr.pix2pix_model.cuda()({"label": torch.zeros(1, 1, 8, 8), "style_image": torch.zeros(1, 4, 1, 8, 8)}, mode="bogus") \
             if torch.cuda.is_available() else (_ for _ in ()).throw(ValueError())
     # the product path never falls back to the CPU
     with pytest.raises(RuntimeError):
@@ -166,14 +168,53 @@ def test_data_parallel_grad_allreduce_gloo_world2():
     assert sorted(res) == [(0, True), (1, True)]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/options"), reason="reference checkout only exists in the build container")
+def test_dropin_trainer_construction_and_checkpoint_layout(tmp_path):
+    """install_dropin() + the reference train.py's construction sequence (import paths, Pix2PixTrainer, save) write
+    checkpoints in the reference's layout."""
+    import pickle
+    import subprocess
+    import sys
+    _, opt = _opts(ngf=8, ndf=8, lambda_l1=10.0)
+    opt.checkpoints_dir, opt.name = str(tmp_path), "dropin"
+    opt_path = tmp_path / "opt.pkl"
+    opt_path.write_bytes(pickle.dumps(opt))
+    code = r'''
+import os, pickle, sys
+sys.path.insert(0, %r)
+sys.dont_write_bytecode = True
+import seg2eye_b200; seg2eye_b200.install_dropin()
+from trainers.pix2pix_trainer import Pix2PixTrainer      # resolves to seg2eye_b200
+import models, models.networks.generator
+assert models.__name__ == "seg2eye_b200.models"
+assert models.networks.generator.__name__ == "seg2eye_b200.models.networks.generator"
+import torch
+from oracle import seg2eye_oracle as O
+opt = pickle.load(open(%r, "rb"))
+tr = Pix2PixTrainer(opt)
+tr.save("latest")
+for label, shapes in (("G", O.generator_shapes(opt)), ("D", O.discriminator_shapes(opt)), ("E", O.encoder_shapes(opt))):
+    sd = torch.load(os.path.join(opt.checkpoints_dir, opt.name, "latest_net_%%s.pth" %% label))
+    assert list(sd) == list(shapes), label
+    for k, v in sd.items():
+        assert tuple(v.shape) == tuple(shapes[k]) and v.device.type == "cpu", (label, k)
+print("DROPIN_OK", type(tr.pix2pix_model).__module__)
+''' % (REPO, str(opt_path))
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
+    assert "DROPIN_OK seg2eye_b200.models.pix2pix_model" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
+
+
+REFERENCE = os.environ.get("S2E_REFERENCE")     # a checkout of the original Seg2Eye project (see oracle/make_golden.py)
+
+
+@pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "options"))),
+                    reason="needs a checkout of the original Seg2Eye project in S2E_REFERENCE")
 def test_reference_option_parsing_and_trainer_construction_with_dropin(tmp_path):
     """The reference's own options package + train.py construction sequence on top of install_dropin()."""
     import subprocess
     import sys
     code = r'''
 import sys, types
-sys.path.insert(0, %r); sys.path.insert(1, "/root/reference")
+sys.path.insert(0, %r); sys.path.insert(1, %r)
 sys.dont_write_bytecode = True
 sys.modules.setdefault("h5py", types.ModuleType("h5py"))
 import cv2; cv2.cv2 = cv2; sys.modules["cv2.cv2"] = cv2
@@ -192,7 +233,7 @@ import os, torch
 sd = torch.load(os.path.join(%r, "dropin", "latest_net_G.pth"))
 assert "head_0.conv_0.weight_orig" in sd and "up_3.norm_s.spade.mlp_gamma.weight" in sd
 print("DROPIN_OK", type(tr.pix2pix_model).__module__)
-''' % (REPO, str(tmp_path), str(tmp_path))
+''' % (REPO, REFERENCE, str(tmp_path), str(tmp_path))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
     assert "DROPIN_OK seg2eye_b200.models.pix2pix_model" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 

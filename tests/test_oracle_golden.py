@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from oracle import seg2eye_oracle as O
+from oracle.make_golden import IMAGE_SUB
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -78,7 +79,9 @@ def test_encoder_generator_discriminator_forward(gold):
         sdG = O.synth_state(O.generator_shapes(opt), seeds["G"])
         taps = {}
         fake = O.generator_forward(sdG, seg, w, opt, taps=taps)
-        close(fake, gold["G_fake"])
+        s, st = sub(fake, IMAGE_SUB)
+        close(s, gold["G_fake_sub"])
+        close(st, gold["G_fake_stat"])
         for name in ("fc", "head_0", "head_0.norm_0", "G_middle_1", "up_0", "up_1", "up_3"):
             t = taps[name]
             if name.endswith("norm_0"):
@@ -118,7 +121,10 @@ def test_two_training_iterations(gold):
             # iteration 1 follows an Adam(beta1=0) update ~ lr*sign(g): fp32 summation-order noise in
             # tiny gradients flips update signs, so near-zero losses (GAN) need an absolute floor
             close(v.detach().reshape(-1), gold["step%d_loss_%s" % (it, k)], 1e-3, atol=0.0 if it == 0 else 5e-4)
-        close(tr.generated, gold["step%d_generated" % it], 1e-3)
+        s, st = sub(tr.generated, IMAGE_SUB)
+        key = "G_fake" if it == 0 else "step%d_generated" % it     # iteration 0 generates G_fake again
+        close(s, gold[key + "_sub"], 1e-3)
+        close(st, gold[key + "_stat"], 1e-3)
     post = dict(G=tr.sdG, D=tr.sdD, E=tr.sdE)
     n = 0
     for k, v in gold.items():
@@ -167,6 +173,7 @@ def test_option_variants_one_iteration(name):
     sds = dict(G=O.synth_state(O.generator_shapes(oopt), SEEDS["G"]), D=O.synth_state(O.discriminator_shapes(oopt), SEEDS["D"]),
                E=O.synth_state(O.encoder_shapes(oopt), SEEDS["E"]))
     batch = O.synth_batch(oopt, 2, SEEDS["batch"])
+    bias0 = sds["D"]["discriminator_1.model4.0.bias"].clone()
     tr = O.OracleTrainer(sds["G"], sds["D"], sds["E"], oopt)
     tr.run_generator_one_step(batch)
     tr.run_discriminator_one_step(batch)
@@ -180,7 +187,14 @@ def test_option_variants_one_iteration(name):
     close(st[:2], ref[name + "|generated_stat"][:2], tol=5e-4)
     close(sds["G"]["conv_img.weight"], ref[name + "|post_G_conv_img.weight"], tol=5e-4)
     close(sds["G"]["up_1.conv_0.weight_u"], ref[name + "|post_G_up_1.conv_0.weight_u"], tol=5e-4)
-    close(sds["D"]["discriminator_1.model4.0.bias"], ref[name + "|post_D_model4_bias"], tol=5e-4, atol=1e-7)
+    bias = sds["D"]["discriminator_1.model4.0.bias"]
+    if oopt.gan_mode == "w":
+        # the Wasserstein loss does not change when every logit shifts by the same constant: the gradient of the logit head's
+        # bias is zero up to summation-order rounding, which Adam's first step (lr * g / (|g| + eps)) turns into any move in
+        # [-lr, lr] (the reference's machine recorded 0.76 lr, another CPU computes g == 0 exactly): only the bound is defined
+        assert float((bias - bias0).abs().max()) <= tr.opt_D.param_groups[0]["lr"] * (1 + 1e-5)
+    else:
+        close(bias, ref[name + "|post_D_model4_bias"], tol=5e-4, atol=1e-7)
 
 
 def _variant2_names():
