@@ -213,6 +213,18 @@ int s2e_norm_stats(const void* x, int B, int HW, int C, int per_sample, double* 
 int s2e_norm_finalize(const double* acc, int G, int C, double count, double count_unbiased, float eps, float* mean,
                       float* rstd, float* running_mean, float* running_var, float momentum,
                       int64_t* num_batches_tracked, void* stream);
+/* Batch statistics shared by several ranks (SyncBatchNorm, normalization.py:72-78 rejects `syncbatch`; the reference SPADE
+ * model's default --norm_G spectralspadesyncbatch3x3 takes them from the vendored sync_batchnorm, batchnorm.py:102-105,
+ * which all-reduces raw sums).  records: double [world][3C + 1], rank r's acc of s2e_norm_stats (G = 1) followed by its
+ * element count n_r (0 for an empty shard).  Combined in rank order with Chan's pairwise update of (mean, M2), never
+ * through raw moments; acc receives the result in the acc format (pivot = global mean, sum (x - p) = 0, sum (x - p)^2 =
+ * M2), count (one double) the total element count. */
+int s2e_norm_merge(const double* records, int world, int C, double* acc, double* count, void* stream);
+/* s2e_norm_finalize (G = 1) with the element count read from the device (`count` of s2e_norm_merge); the unbiased
+ * running_var correction uses count * unbiased_factor (4 when the statistics come from a nearest-2x up-sampling's source). */
+int s2e_norm_finalize_merged(const double* acc, const double* count, int C, double unbiased_factor, float eps, float* mean,
+                             float* rstd, float* running_mean, float* running_var, float momentum,
+                             int64_t* num_batches_tracked, void* stream);
 /* act_mask (nullable): one BIT per element, [B*HW][C/8] bytes, bit j of byte (p, c/8) = (out[p][c+j] > 0); all the
  * backward pass needs to know about `out` (read instead of it: 0.125 B/element instead of 2). */
 /* up_w != 0: x is the [B][H/2][W/2][C] tensor whose nearest-2x up-sampling (generator.py:50) is the block input; up_w = W
@@ -228,7 +240,7 @@ int s2e_spade_params(const float* mean, const float* rstd, const float* style, i
 int s2e_spade_style_fwd(const void* x, const void* gb, const float* style, const float* mean, const float* rstd,
                         int B, int HW, int C, int per_sample, int act, void* out, uint8_t* act_mask, int up_w,
                         void* stream);
-/* backward: racc = scratch of B*5*C doubles + B*2*C floats, zeroed inside. `act_mask` = the forward pass's mask (may be
+/* backward: racc = scratch of B*5*C doubles + B*2*C floats + 2*C + 1 doubles, zeroed inside. `act_mask` = the forward pass's mask (may be
  * NULL when act == NONE).  chsum (nullable, float [3][C]) receives the per-channel sums over the batch of dgamma, dbeta
  * and dx -- the bias gradients of the gamma|beta convolution (normalization.py:88-89) and of the convolution that
  * produced x (architecture.py:24) -- which the statistics pass yields for free.  dx_accumulate != 0 adds into dx
@@ -241,6 +253,23 @@ int s2e_spade_style_bwd(const void* dout, const uint8_t* act_mask, const void* x
                         double* racc, void* dx, int dx_accumulate, void* dgb, float* dstyle, float* chsum, int up_w,
                         int gb_stride /* channels per pixel of `gb`: 0 = 2C (gamma|beta); C when only gamma was kept */,
                         void* stream);
+/* s2e_spade_style_bwd in two halves, so that ranks sharing batch statistics can add their per-channel sums in between
+ * (normalization.py:75 with SyncBatchNorm: the statistics, hence their gradient terms, span the global batch).
+ * reduce: the raw-moment pass and the fold; dstyle and chsum as above (chsum's third row relies on the normalisation
+ * part of dx summing to zero, which under shared statistics holds over the global batch only: a rank's value is off by
+ * its share, and the shares cancel when the bias gradients are summed across ranks).  For batch statistics (bit 0 of
+ * per_sample clear) sums = double [2][C] + 1: S1 = sum dxhat, S2 = sum dxhat * xhat per channel and this call's element
+ * count B*HW; per-sample statistics keep theirs in racc.  racc = scratch of B*5*C doubles + B*2*C floats.
+ * apply: dx / dgamma|dbeta from racc and sums, whose S1, S2 and count may have been summed over ranks (m1 = S1 / count,
+ * m2 = S2 / count).  Running the two back to back is s2e_spade_style_bwd, bit for bit. */
+int s2e_spade_style_bwd_reduce(const void* dout, const uint8_t* act_mask, const void* x, const void* gb, const float* style,
+                               const float* mean, const float* rstd, int B, int HW, int C, int per_sample, int act,
+                               double* racc, double* sums, float* dstyle, float* chsum, int up_w, int gb_stride,
+                               void* stream);
+int s2e_spade_style_bwd_apply(const void* dout, const uint8_t* act_mask, const void* x, const void* gb, const float* style,
+                              const float* mean, const float* rstd, int B, int HW, int C, int per_sample, int act,
+                              const double* racc, const double* sums, void* dx, int dx_accumulate, void* dgb, int up_w,
+                              int gb_stride, void* stream);
 
 /* InstanceNorm2d(affine=False)+optional LeakyReLU on NHWC bf16 (normalization.py:41; discriminator.py:88-92;
  * encoder.py:23-38).  in_scale (nullable): one factor per `group` consecutive images, applied to x implicitly. */

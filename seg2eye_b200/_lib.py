@@ -66,9 +66,13 @@ _SIGS = {
     "s2e_depth_to_space": [_P, _I, _I, _I, _I, _P, _P],
     "s2e_norm_stats": [_P, _I, _I, _I, _I, _P, _P],
     "s2e_norm_finalize": [_P, _I, _I, _D, _D, _F, _P, _P, _P, _P, _F, _P, _P],
+    "s2e_norm_merge": [_P, _I, _I, _P, _P, _P],
+    "s2e_norm_finalize_merged": [_P, _P, _I, _D, _F, _P, _P, _P, _P, _F, _P, _P],
     "s2e_spade_params": [_P, _P, _P, _I, _I, _I, _P, _P],
     "s2e_spade_style_fwd": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P],
     "s2e_spade_style_bwd": [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P, _P, _I, _I, _P],
+    "s2e_spade_style_bwd_reduce": [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _I, _I, _P],
+    "s2e_spade_style_bwd_apply": [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _I, _P, _I, _I, _P],
     "s2e_instnorm_fwd": [_P, _I, _I, _I, _I, _F, _P, _I, _P, _P, _P, _P, _P, _P],
     "s2e_instnorm_bwd": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P],
     "s2e_upsample2x_fwd": [_P, _I, _I, _I, _I, _P, _P],

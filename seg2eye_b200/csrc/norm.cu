@@ -86,12 +86,19 @@ __global__ void __launch_bounds__(NT) stats_kernel(const bf16* __restrict__ x, i
 
 // in_scale (optional, one value per `group` consecutive statistic groups): statistics are those of x * in_scale without
 // the product ever being formed: mean stays that of x, rstd' = s / sqrt(var * s^2 + eps), so (x - mean) * rstd' == norm(s x).
+// count_dev (optional): the element count lives on the device (statistics merged across ranks, s2e_norm_merge); then
+// count = count_dev[0] and count_unbiased = count_dev[0] * count_unbiased (the host passes the up-sampling factor).
 __global__ void finalize_kernel(const double* __restrict__ acc, int G, int C, double count, float eps, float* mean,
                                 float* rstd, float* running_mean, float* running_var, float momentum,
-                                long long* nbt, const float* __restrict__ in_scale, int group, double count_unbiased) {
+                                long long* nbt, const float* __restrict__ in_scale, int group, double count_unbiased,
+                                const double* __restrict__ count_dev = nullptr) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0 && nbt) *nbt += 1;
   if (i >= G * C) return;
+  if (count_dev) {
+    count = count_dev[0];
+    count_unbiased *= count;
+  }
   const int g = i / C, c = i % C;
   const double s = acc[(size_t)g * 3 * C + c], ss = acc[(size_t)g * 3 * C + C + c], pivot = acc[(size_t)g * 3 * C + 2 * (size_t)C + c];
   const double ms = s / count;          // mean of the shifted data
@@ -107,6 +114,37 @@ __global__ void finalize_kernel(const double* __restrict__ acc, int G, int C, do
     running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)m;
     running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unb;
   }
+}
+
+// Statistics of several ranks (or batch shards) combined into one record: rec[r] = [sum (x-p_r)][sum (x-p_r)^2][p_r] (C each,
+// the acc format of stats_kernel) followed by the element count n_r.  Chan et al.'s pairwise update in rank order,
+//   mean_r = p_r + s_r / n_r,  M2_r = ss_r - s_r^2 / n_r,  delta = mean_r - mean,
+//   mean += delta n_r / (n + n_r),  M2 += M2_r + delta^2 n n_r / (n + n_r),
+// never forms raw moments, so a channel whose mean is large against its spread, or shards whose means differ by many
+// sigma, lose no precision.  Output in the acc format (pivot = global mean, sum (x - p) = 0, sum (x - p)^2 = M2) and the
+// total count.  Empty shards (n_r = 0) are skipped.
+__global__ void merge_kernel(const double* __restrict__ rec, int world, int C, double* __restrict__ acc,
+                             double* __restrict__ count) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  const size_t stride = 3 * (size_t)C + 1;
+  double n = 0, mean = 0, m2 = 0;
+  for (int r = 0; r < world; ++r) {
+    const double* q = rec + r * stride;
+    const double nr = q[3 * (size_t)C];
+    if (nr <= 0) continue;
+    const double s = q[c], ss = q[C + c];
+    const double mr = q[2 * (size_t)C + c] + s / nr;
+    const double m2r = fmax(ss - s * s / nr, 0.0);
+    const double tot = n + nr, d = mr - mean;
+    mean = n == 0 ? mr : mean + d * (nr / tot);
+    m2 = n == 0 ? m2r : m2 + m2r + d * d * (n * nr / tot);
+    n = tot;
+  }
+  acc[c] = 0.0;
+  acc[C + c] = m2;
+  acc[2 * (size_t)C + c] = mean;
+  if (c == 0) *count = n;
 }
 
 // Pixel index of x for output pixel q of sample b.  up_w == 0: x has the output's resolution.  up_w = W of the output:
@@ -370,12 +408,16 @@ __global__ void __launch_bounds__(NT) spade_bwd_reduce_kernel(const bf16* __rest
   block_channel_reduce_u<4, UP ? 1 : 4>(C, u0, u1, racc + (size_t)b * 5 * C, body);
 }
 
-// fold: raw moments -> m1 / m2 per statistics group (float [G][2][C]), dstyle [B][2C] and, optionally, chsum [3][C] =
+// fold: raw moments -> per-sample statistics m1 / m2 (float [B][2][C]) or, for batch statistics, the per-channel sums
+// S1 = sum dxh, S2 = sum dxh xh and their element count (double [2][C] + 1: `sums`, turned into m1 / m2 by the apply pass,
+// so that ranks sharing batch statistics can add their sums in between), dstyle [B][2C] and, optionally, chsum [3][C] =
 // per-channel sums over the whole batch of dgamma, dbeta and dx.  The last one needs no extra pass: the normalisation part
-// of dx sums to zero over the pixels its statistics were taken from, so sum dx = sum_b (1 + s0[b]) * T1[b].
+// of dx sums to zero over the pixels its statistics were taken from, so sum dx = sum_b (1 + s0[b]) * T1[b].  With
+// statistics shared across ranks that holds over the global batch only; a rank's sum is then off by its share of the
+// normalisation part, but the bias gradients it feeds are summed across ranks before use, and the shares cancel there.
 __global__ void spade_style_bwd_fold_kernel(const double* __restrict__ racc, int B, int C, int per_sample, int frozen, double count,
                                             const float* __restrict__ style, const float* __restrict__ mean,
-                                            const float* __restrict__ rstd, float* __restrict__ m12,
+                                            const float* __restrict__ rstd, float* __restrict__ m12, double* __restrict__ sums,
                                             float* __restrict__ dstyle, float* __restrict__ chsum) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * C) return;
@@ -406,8 +448,9 @@ __global__ void spade_style_bwd_fold_kernel(const double* __restrict__ racc, int
       if (style) sx += (1.0 + (double)style[(size_t)bb * 2 * C + c]) * t1;
     }
     if (!per_sample) {
-      m12[c] = frozen ? 0.f : (float)(s1 / count);
-      m12[C + c] = frozen ? 0.f : (float)(s2 / count);
+      sums[c] = s1;
+      sums[C + c] = s2;
+      if (c == 0) sums[2 * (size_t)C] = count;
     }
     if (chsum) {
       chsum[c] = (float)sg;
@@ -423,7 +466,8 @@ template <int ACT, bool UP>
 __global__ void __launch_bounds__(NT) spade_bwd_apply_kernel(const bf16* __restrict__ dout, const uint8_t* __restrict__ amask,
                                                              const bf16* __restrict__ x, const bf16* __restrict__ gb,
                                                              const float* __restrict__ style, const float* __restrict__ mean,
-                                                             const float* __restrict__ rstd, const float* __restrict__ m12, int HW,
+                                                             const float* __restrict__ rstd, const float* __restrict__ m12,
+                                                             const double* __restrict__ sums, int frozen, int HW,
                                                              int C, int per_sample, bf16* __restrict__ dx, int dx_acc,
                                                              bf16* __restrict__ dgb, int W, int gstride) {
   const int b = blockIdx.y;
@@ -448,7 +492,15 @@ __global__ void __launch_bounds__(NT) spade_bwd_apply_kernel(const bf16* __restr
     float kA[8], kR[8], kC[8], kD[8], kE[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
-      const float rs = rstd[so + c + j], mu = mean[so + c + j], m1 = m1p[c + j], m2 = m1p[C + c + j];
+      float m1, m2;
+      if (per_sample) {
+        m1 = m1p[c + j];
+        m2 = m1p[C + c + j];
+      } else {    // batch statistics: from this batch's sums, or those of all ranks added together
+        m1 = frozen ? 0.f : (float)(sums[c + j] / sums[2 * (size_t)C]);
+        m2 = frozen ? 0.f : (float)(sums[C + c + j] / sums[2 * (size_t)C]);
+      }
+      const float rs = rstd[so + c + j], mu = mean[so + c + j];
       kR[j] = rs;
       kA[j] = rs + (s0p ? 1.f + s0p[c + j] : 0.f);
       kC[j] = -rs * rs * m2;
@@ -803,6 +855,7 @@ int s2e_norm_stats(const void* x, int B, int HW, int C, int per_sample, double* 
   cudaStream_t st = (cudaStream_t)stream;
   const int G = per_sample ? B : 1;
   S2E_CHECK_CUDA(cudaMemsetAsync(acc, 0, sizeof(double) * G * 3 * C, st));   // [sum (x-p)][sum (x-p)^2][pivot p] per group
+  if ((long long)B * HW == 0) return S2E_OK;    // an empty batch (shard): zero sums, no pivot pixel to read
   const long long span = per_sample ? HW : (long long)B * HW;
   dim3 grid(red_chunks(span, G), G);
   stats_kernel<<<grid, NT, red_smem(C), st>>>((const bf16*)x, HW, C, (long long)B * HW, per_sample, acc);
@@ -815,6 +868,22 @@ int s2e_norm_finalize(const double* acc, int G, int C, double count, double coun
   finalize_kernel<<<ceil_div(G * C, 256), 256, 0, (cudaStream_t)stream>>>(acc, G, C, count, eps, mean, rstd, running_mean,
                                                                            running_var, momentum, (long long*)nbt, nullptr, 1,
                                                                            count_unbiased);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+
+int s2e_norm_merge(const double* records, int world, int C, double* acc, double* count, void* stream) {
+  S2E_REQUIRE(world >= 1 && C >= 1, "norm_merge: bad world %d / C %d", world, C);
+  merge_kernel<<<ceil_div(C, 256), 256, 0, (cudaStream_t)stream>>>(records, world, C, acc, count);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+
+int s2e_norm_finalize_merged(const double* acc, const double* count, int C, double unbiased_factor, float eps, float* mean,
+                             float* rstd, float* running_mean, float* running_var, float momentum, int64_t* nbt, void* stream) {
+  finalize_kernel<<<ceil_div(C, 256), 256, 0, (cudaStream_t)stream>>>(acc, 1, C, 0.0, eps, mean, rstd, running_mean, running_var,
+                                                                      momentum, (long long*)nbt, nullptr, 1, unbiased_factor,
+                                                                      count);
   S2E_LAUNCH_CHECK();
   return S2E_OK;
 }
@@ -882,28 +951,53 @@ int s2e_spade_style_fwd(const void* x, const void* gb, const float* style, const
   return S2E_OK;
 }
 
-int s2e_spade_style_bwd(const void* dout, const uint8_t* act_mask, const void* x, const void* gb, const float* style,
-                        const float* mean, const float* rstd, int B, int HW, int C, int per_sample, int act, double* racc,
-                        void* dx, int dx_accumulate, void* dgb, float* dstyle, float* chsum, int up_w, int gb_stride,
-                        void* stream) {
+// ACT_ / UP_ dispatch of the SPADE+Style backward kernels
+#define S2E_SPADE_BWD_DISPATCH(M)                        \
+  do {                                                   \
+    if (up_w) {                                          \
+      if (act == S2E_ACT_LRELU) M(S2E_ACT_LRELU, true);  \
+      else if (act == S2E_ACT_RELU) M(S2E_ACT_RELU, true); \
+      else M(S2E_ACT_NONE, true);                        \
+    } else {                                             \
+      if (act == S2E_ACT_LRELU) M(S2E_ACT_LRELU, false); \
+      else if (act == S2E_ACT_RELU) M(S2E_ACT_RELU, false); \
+      else M(S2E_ACT_NONE, false);                       \
+    }                                                    \
+  } while (0)
+
+static int spade_bwd_check(const uint8_t* act_mask, const float* style, const float* dstyle, int HW, int C, int act, int up_w,
+                           int gb_stride) {
   S2E_REQUIRE(C % 8 == 0, "spade_style_bwd needs C %% 8 == 0 (C=%d)", C);
   S2E_REQUIRE(up_w == 0 || (up_w % 2 == 0 && HW % up_w == 0 && (HW / up_w) % 2 == 0), "spade_style_bwd: bad up-sampled width %d", up_w);
-  cudaStream_t st = (cudaStream_t)stream;
-  // racc: double [B][5][C] followed by float m12 [B][2][C]
   S2E_REQUIRE(act == S2E_ACT_NONE || act_mask, "spade_style_bwd: the activation mask written by the forward pass is required");
   const int gstride = gb_stride > 0 ? gb_stride : 2 * C;
   S2E_REQUIRE(gstride >= C && gstride % 8 == 0, "spade_style_bwd: bad gamma stride %d", gstride);
   S2E_REQUIRE(style || !dstyle, "spade_style_bwd: plain SPADE (style == NULL) has no style gradient");
+  return S2E_OK;
+}
+
+int s2e_spade_style_bwd_reduce(const void* dout, const uint8_t* act_mask, const void* x, const void* gb, const float* style,
+                               const float* mean, const float* rstd, int B, int HW, int C, int per_sample, int act,
+                               double* racc, double* sums, float* dstyle, float* chsum, int up_w, int gb_stride, void* stream) {
+  S2E_REQUIRE((per_sample & 1) || sums, "spade_style_bwd_reduce: batch statistics need the `sums` buffer");
+  cudaStream_t st = (cudaStream_t)stream;
+  if ((long long)B * HW == 0) {   // an empty shard (its tensors may be NULL) adds nothing to the sums of its peers
+    if (!(per_sample & 1)) S2E_CHECK_CUDA(cudaMemsetAsync(sums, 0, sizeof(double) * (2 * C + 1), st));
+    return S2E_OK;
+  }
+  int rc = spade_bwd_check(act_mask, style, dstyle, HW, C, act, up_w, gb_stride);
+  if (rc) return rc;
+  // racc: double [B][5][C] followed by float m12 [B][2][C]
   S2E_CHECK_CUDA(cudaMemsetAsync(racc, 0, sizeof(double) * B * 5 * C, st));
   float* m12 = (float*)(racc + (size_t)B * 5 * C);
   // per_sample bit 1: the statistics are constants (BatchNorm in eval mode: running statistics) -- no m1 / m2 terms
   const int frozen = (per_sample >> 1) & 1;
   per_sample &= 1;
+  const int gstride = gb_stride > 0 ? gb_stride : 2 * C;
   const float os = style ? 0.5f : 1.0f;
   const int units = up_w ? HW / 4 : HW;     // source pixels when the up-sampling is folded in
-  dim3 grid2(ew_chunks(units, B, C), B);
   const double count = per_sample ? (double)HW : (double)B * HW;
-#define S2E_SPADE_BWD(ACT_, UP_)                                                                                              \
+#define S2E_SPADE_BWD_REDUCE(ACT_, UP_)                                                                                       \
   do {                                                                                                                        \
     /* the reduce pass runs as exactly ONE wave of resident blocks (its register count differs per instantiation) */        \
     int nb = 2;                                                                                                               \
@@ -912,26 +1006,53 @@ int s2e_spade_style_bwd(const void* dout, const uint8_t* act_mask, const void* x
     spade_bwd_reduce_kernel<ACT_, UP_><<<grid, NT, red_smem(C), st>>>((const bf16*)dout, act_mask, (const bf16*)x, (const bf16*)gb, \
                                                                       HW, C, racc, up_w, gstride, os);                        \
     S2E_LAUNCH_CHECK();                                                                                                       \
-    spade_style_bwd_fold_kernel<<<ceil_div(B * C, 256), 256, 0, st>>>(racc, B, C, per_sample, frozen, count, style, mean, rstd, m12, \
-                                                                      dstyle, chsum);                                         \
-    S2E_LAUNCH_CHECK();                                                                                                       \
-    spade_bwd_apply_kernel<ACT_, UP_><<<grid2, NT, 0, st>>>((const bf16*)dout, act_mask, (const bf16*)x, (const bf16*)gb, style, \
-                                                            mean, rstd, m12, HW, C, per_sample, (bf16*)dx, dx_accumulate,     \
-                                                            (bf16*)dgb, up_w, gstride);                                       \
-    S2E_LAUNCH_CHECK();                                                                                                       \
   } while (0)
-  if (up_w) {
-    if (act == S2E_ACT_LRELU) S2E_SPADE_BWD(S2E_ACT_LRELU, true);
-    else if (act == S2E_ACT_RELU) S2E_SPADE_BWD(S2E_ACT_RELU, true);
-    else S2E_SPADE_BWD(S2E_ACT_NONE, true);
-  } else {
-    if (act == S2E_ACT_LRELU) S2E_SPADE_BWD(S2E_ACT_LRELU, false);
-    else if (act == S2E_ACT_RELU) S2E_SPADE_BWD(S2E_ACT_RELU, false);
-    else S2E_SPADE_BWD(S2E_ACT_NONE, false);
-  }
-#undef S2E_SPADE_BWD
+  S2E_SPADE_BWD_DISPATCH(S2E_SPADE_BWD_REDUCE);
+#undef S2E_SPADE_BWD_REDUCE
+  spade_style_bwd_fold_kernel<<<ceil_div(B * C, 256), 256, 0, st>>>(racc, B, C, per_sample, frozen, count, style, mean, rstd, m12,
+                                                                    sums, dstyle, chsum);
+  S2E_LAUNCH_CHECK();
   return S2E_OK;
 }
+
+int s2e_spade_style_bwd_apply(const void* dout, const uint8_t* act_mask, const void* x, const void* gb, const float* style,
+                              const float* mean, const float* rstd, int B, int HW, int C, int per_sample, int act,
+                              const double* racc, const double* sums, void* dx, int dx_accumulate, void* dgb, int up_w,
+                              int gb_stride, void* stream) {
+  if ((long long)B * HW == 0) return S2E_OK;
+  int rc = spade_bwd_check(act_mask, style, nullptr, HW, C, act, up_w, gb_stride);
+  if (rc) return rc;
+  S2E_REQUIRE((per_sample & 1) || sums, "spade_style_bwd_apply: batch statistics need the `sums` buffer");
+  cudaStream_t st = (cudaStream_t)stream;
+  const float* m12 = (const float*)(racc + (size_t)B * 5 * C);
+  const int frozen = (per_sample >> 1) & 1;
+  per_sample &= 1;
+  const int gstride = gb_stride > 0 ? gb_stride : 2 * C;
+  const int units = up_w ? HW / 4 : HW;
+  dim3 grid2(ew_chunks(units, B, C), B);
+#define S2E_SPADE_BWD_APPLY(ACT_, UP_)                                                                                        \
+  spade_bwd_apply_kernel<ACT_, UP_><<<grid2, NT, 0, st>>>((const bf16*)dout, act_mask, (const bf16*)x, (const bf16*)gb, style, \
+                                                          mean, rstd, m12, sums, frozen, HW, C, per_sample, (bf16*)dx,        \
+                                                          dx_accumulate, (bf16*)dgb, up_w, gstride)
+  S2E_SPADE_BWD_DISPATCH(S2E_SPADE_BWD_APPLY);
+#undef S2E_SPADE_BWD_APPLY
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+
+int s2e_spade_style_bwd(const void* dout, const uint8_t* act_mask, const void* x, const void* gb, const float* style,
+                        const float* mean, const float* rstd, int B, int HW, int C, int per_sample, int act, double* racc,
+                        void* dx, int dx_accumulate, void* dgb, float* dstyle, float* chsum, int up_w, int gb_stride,
+                        void* stream) {
+  // racc: double [B][5][C], float m12 [B][2][C], then the batch-statistics sums, double [2][C] + 1
+  double* sums = racc + (size_t)B * 5 * C + (size_t)B * C;
+  int rc = s2e_spade_style_bwd_reduce(dout, act_mask, x, gb, style, mean, rstd, B, HW, C, per_sample, act, racc, sums, dstyle,
+                                      chsum, up_w, gb_stride, stream);
+  if (rc) return rc;
+  return s2e_spade_style_bwd_apply(dout, act_mask, x, gb, style, mean, rstd, B, HW, C, per_sample, act, racc, sums, dx,
+                                   dx_accumulate, dgb, up_w, gb_stride, stream);
+}
+#undef S2E_SPADE_BWD_DISPATCH
 
 int s2e_sn_in_correction(const double* racc, const float* rstd, const float* inv_sigma, int Bn, int group, int C, float eps,
                          const float* U, const float* V, int K, float* coef, float* dw, void* stream) {

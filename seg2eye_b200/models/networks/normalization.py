@@ -130,7 +130,10 @@ class SPADE(nn.Module):
         if param_free_norm_type == 'instance':
             self.param_free_norm = InstanceNorm2d(norm_nc)
             self.per_sample = True
-        elif param_free_norm_type == 'batch':
+        elif param_free_norm_type in ('batch', 'syncbatch'):
+            # syncbatch (the reference SPADE's default, rejected by Seg2Eye): torch.nn.SyncBatchNorm(affine=False) --
+            # training-mode statistics of the global batch across the ranks of the default process group; the same
+            # buffers (and state_dict) as batch, and the same computation with one rank or in eval mode
             self.param_free_norm = BatchNorm2dStats(norm_nc)
             self.per_sample = False
         else:
@@ -141,6 +144,7 @@ class SPADE(nn.Module):
         self.mlp_gamma = Conv2d(nhidden, norm_nc, ks, padding=pw)
         self.mlp_beta = Conv2d(nhidden, norm_nc, ks, padding=pw)
         self.norm_nc = norm_nc
+        self.sync = param_free_norm_type == 'syncbatch'
 
     def _actv(self, segmap, h, w):
         """ReLU(mlp_shared(nearest(segmap))) and whether its ReLU backward is left to the gamma|beta data gradient."""
@@ -169,7 +173,7 @@ class SPADE(nn.Module):
         if up:
             H, W = 2 * H, 2 * W
         pfn = self.param_free_norm
-        cfg = ops.NormCfg(self.per_sample, act, self.training, 0.1, 1e-5)
+        cfg = ops.NormCfg(self.per_sample, act, self.training, 0.1, 1e-5, self.sync)
         bufs = (None, None, None) if self.per_sample else (pfn.running_mean, pfn.running_var, pfn.num_batches_tracked)
         if not torch.is_grad_enabled() and ops.spade_conv_fused_ok(x, up, self.mlp_gamma.in_channels):
             # no autograd graph wanted (D step's generator pass, inference): gamma|beta are consumed in the epilogue of

@@ -12,6 +12,7 @@ from collections import namedtuple
 import torch
 
 from . import _lib as L
+from . import parallel
 
 BF16 = torch.bfloat16
 F32 = torch.float32
@@ -630,7 +631,8 @@ def prepare_spectral(convs, training, n_calls=1, keep_uv=False):
 
 
 # ------------------------------------------------------------------------------------------------ norms
-NormCfg = namedtuple("NormCfg", "per_sample act training momentum eps")
+# sync: BatchNorm statistics shared by all ranks of the default process group (SyncBatchNorm, `spadesyncbatch`)
+NormCfg = namedtuple("NormCfg", "per_sample act training momentum eps sync", defaults=(False,))
 
 
 _stats_memo = {"ref": None, "key": None, "acc": None}
@@ -638,6 +640,31 @@ _stats_memo = {"ref": None, "key": None, "acc": None}
 
 def clear_stats_memo():
     _stats_memo["ref"] = _stats_memo["key"] = _stats_memo["acc"] = None
+
+
+def synced(cfg):
+    """Whether a normalisation with this config takes the statistics of the global batch over several ranks: BatchNorm
+    statistics in training mode under a process group of more than one rank.  Every rank must then run the same
+    training-mode forwards (and their backwards) in the same order -- each one issues a collective, as with
+    torch.nn.SyncBatchNorm -- on the default (NCCL) group, interleaved with the gradient all-reduces."""
+    return cfg.sync and cfg.training and not cfg.per_sample and parallel.world_size() > 1
+
+
+def _merged_record(x):
+    """acc and element count (device, fp64) of x's statistics over the global batch: every rank's s2e_norm_stats record and
+    count are all-gathered, then combined by s2e_norm_merge."""
+    B, Hx, Wx, Cc = x.shape
+    st = L.stream()
+    rec = torch.empty(3 * Cc + 1, dtype=torch.float64, device=x.device)
+    L.call("s2e_norm_stats", L.ptr(x), B, Hx * Wx, Cc, 0, L.ptr(rec), st)
+    rec[3 * Cc:].fill_(float(B * Hx * Wx))      # elements summed (the source's, when x is up-sampled)
+    world = parallel.world_size()
+    recs = torch.empty(world * (3 * Cc + 1), dtype=torch.float64, device=x.device)
+    torch.distributed.all_gather_into_tensor(recs, rec)
+    acc = torch.empty(3 * Cc, dtype=torch.float64, device=x.device)
+    count = torch.empty(1, dtype=torch.float64, device=x.device)
+    L.call("s2e_norm_merge", L.ptr(recs), world, Cc, L.ptr(acc), L.ptr(count), st)
+    return acc, count
 
 
 def spade_statistics(x, cfg, running_mean, running_var, nbt, up):
@@ -657,16 +684,27 @@ def spade_statistics(x, cfg, running_mean, running_var, nbt, up):
     count = float(H * W if cfg.per_sample else B * H * W)     # elements BatchNorm sees (unbiased running_var)
     count_stats = count / 4 if up else count                  # elements actually summed (the 4x smaller source)
     # norm_s and norm_0 of a block with a learned shortcut normalise the SAME tensor (architecture.py:44-49): the sums are
-    # taken once, each layer finalises them into its own mean / rstd / running buffers
+    # taken once (with shared statistics: merged across ranks once, one collective), each layer finalises them into its
+    # own mean / rstd / running buffers
+    sync = synced(cfg)
     memo = _stats_memo
-    key = (x.data_ptr(), x._version, tuple(x.shape), int(cfg.per_sample))
+    key = (x.data_ptr(), x._version, tuple(x.shape), int(cfg.per_sample), sync)
     if memo["ref"] is not None and memo["ref"]() is not None and memo["key"] == key:   # the summed tensor is still alive: same data
         acc = memo["acc"]
         _state["stats_shared"] = _state.get("stats_shared", 0) + 1
+    elif sync:
+        acc = _merged_record(x)
+        _state["sync_collectives"] = _state.get("sync_collectives", 0) + 1
+        memo["ref"], memo["key"], memo["acc"] = _weakref.ref(x), key, acc
     else:
         acc = torch.empty(G * 3 * Cc, dtype=torch.float64, device=x.device)    # [sum (x-p)][sum (x-p)^2][pivot p] per group
         L.call("s2e_norm_stats", L.ptr(x), B, Hx * Wx, Cc, int(cfg.per_sample), L.ptr(acc), st)
         memo["ref"], memo["key"], memo["acc"] = _weakref.ref(x), key, acc
+    if sync:
+        acc, n = acc
+        L.call("s2e_norm_finalize_merged", L.ptr(acc), L.ptr(n), Cc, 4.0 if up else 1.0, cfg.eps, L.ptr(mean), L.ptr(rstd),
+               L.ptr(running_mean), L.ptr(running_var), cfg.momentum, L.ptr(nbt), st)
+        return mean, rstd, True
     L.call("s2e_norm_finalize", L.ptr(acc), G, Cc, count_stats, count, cfg.eps, L.ptr(mean), L.ptr(rstd),
            L.ptr(running_mean) if upd else None, L.ptr(running_var) if upd else None, cfg.momentum,
            L.ptr(nbt) if upd else None, st)
@@ -726,6 +764,30 @@ class GradSink:
         self.buf, self.users, self.seen = None, 0, 0
 
 
+def _spade_style_bwd(synced, dout, amask, x, gb, style, mean, rstd, B, HW, Cc, stat_mode, act, dx, accumulate, dgb, dstyle, chsum,
+                     up_w, gb_stride, tag):
+    """s2e_spade_style_bwd; with statistics shared across ranks (`synced`), its two halves with the all-reduce of the
+    per-channel sums S1, S2 and of the element count between them, so that dx is the gradient of the global-batch
+    normalisation.  The 1/world_size factor that the multi-rank graph step puts on the loss is the same on every rank: it
+    scales every rank's S1, S2 alike, and S / (global count) stays consistent with the loss that is differentiated."""
+    st = L.stream()
+    # double [B][5][C], float m12 [B][2][C], then the batch-statistics sums double [2][C] + 1
+    racc = torch.empty(B * 5 * Cc + B * Cc + 2 * Cc + 1, dtype=torch.float64, device=x.device)
+    args = (L.ptr(dout), L.ptr(amask), L.ptr(x), L.ptr(gb), L.ptr(style), L.ptr(mean), L.ptr(rstd), B, HW, Cc, stat_mode, act,
+            L.ptr(racc))
+    if not synced:
+        _timed_call("normb", 12.0 * B * HW * Cc, "s2e_spade_style_bwd", *args, L.ptr(dx), int(accumulate), L.ptr(dgb),
+                    L.ptr(dstyle), L.ptr(chsum), up_w, gb_stride, st, tag=tag)
+        return
+    sums = racc[B * 6 * Cc:]
+    _timed_call("normb", 4.0 * B * HW * Cc, "s2e_spade_style_bwd_reduce", *args, L.ptr(sums), L.ptr(dstyle), L.ptr(chsum),
+                up_w, gb_stride, st, tag=tag + " reduce")
+    torch.distributed.all_reduce(sums)
+    _state["sync_collectives"] = _state.get("sync_collectives", 0) + 1
+    _timed_call("normb", 8.0 * B * HW * Cc, "s2e_spade_style_bwd_apply", *args, L.ptr(sums), L.ptr(dx), int(accumulate),
+                L.ptr(dgb), up_w, gb_stride, st, tag=tag + " apply")
+
+
 class SpadeStyleFn(torch.autograd.Function):
     """out = act(0.5 * [ norm(x) * (1 + gamma) + beta + x * (1 + s0) + s1 ])  (normalization.py:91-105,161-192).
 
@@ -754,7 +816,7 @@ class SpadeStyleFn(torch.autograd.Function):
         _timed_call("norm", 8.0 * B * H * W * Cc, "s2e_spade_style_fwd", L.ptr(x), L.ptr(gb), L.ptr(style), L.ptr(mean),
                     L.ptr(rstd), B, H * W, Cc, int(cfg.per_sample), cfg.act, L.ptr(out), L.ptr(amask), W if up else 0, st,
                     tag="B%d HW%d C%d%s" % (B, H * W, Cc, " up" if up else ""))
-        ctx.cfg, ctx.batch_stats, ctx.hw = cfg, batch_stats, (H, W)
+        ctx.cfg, ctx.batch_stats, ctx.hw, ctx.synced = cfg, batch_stats, (H, W), synced(cfg)
         ctx.save_for_backward(x, gb, style, mean, rstd, amask)
         return out
 
@@ -765,8 +827,6 @@ class SpadeStyleFn(torch.autograd.Function):
         dout = _c(dout)
         B, Cc = x.shape[0], x.shape[3]
         H, W = ctx.hw
-        st = L.stream()
-        racc = torch.empty(B * 5 * Cc + (B * 2 * Cc + 1) // 2, dtype=torch.float64, device=x.device)
         accumulate = sink is not None and sink.buf is not None
         # gradient w.r.t. x itself: with `up` the kernel adds the four output pixels of every source pixel on the spot (the
         # adjoint of the nearest-2x up-sampling), so the full-resolution gradient is never written
@@ -783,9 +843,8 @@ class SpadeStyleFn(torch.autograd.Function):
         chsum = torch.empty(3 * Cc, dtype=F32, device=x.device)
         # eval-mode BatchNorm (running statistics): the statistics are constants, bit 1 of the per_sample argument says so
         stat_mode = int(cfg.per_sample) | (0 if ctx.batch_stats else 2)
-        _timed_call("normb", 12.0 * B * H * W * Cc, "s2e_spade_style_bwd", L.ptr(dout), L.ptr(amask), L.ptr(x), L.ptr(gb), L.ptr(style), L.ptr(mean),
-                    L.ptr(rstd), B, H * W, Cc, stat_mode, cfg.act, L.ptr(racc), L.ptr(dx), int(accumulate), L.ptr(dgb),
-                    L.ptr(dstyle), L.ptr(chsum), W if up else 0, 0, st, tag="bwd B%d HW%d C%d%s" % (B, H * W, Cc, " up" if up else ""))
+        _spade_style_bwd(ctx.synced, dout, amask, x, gb, style, mean, rstd, B, H * W, Cc, stat_mode, cfg.act, dx, accumulate, dgb,
+                         dstyle, chsum, W if up else 0, 0, "bwd B%d HW%d C%d%s" % (B, H * W, Cc, " up" if up else ""))
         # per-channel sums of the two gradients, for the bias gradients of the convolutions that receive them as dy
         # (TapConvFn.backward picks the attribute up when the tensor reaches it unmodified; otherwise it sums itself)
         dgb._s2e_chsum, dgb._s2e_chsum_ver = chsum[:2 * Cc], (dgb._version, dgb.data_ptr())
@@ -856,7 +915,7 @@ class SpadeConvFn(torch.autograd.Function):
         flops = 2.0 * B * H * W * 2 * Cc * Ca * conv_cfg.kh * conv_cfg.kw
         _timed_call("tc", flops, "s2e_tapconv_fwd", d, L.ptr(actv), L.ptr(wp), L.ptr(bias), None, L.ptr(out), L.IMPL_TC, st,
                     tag="fwd+spade B%d %dx%d Cin%d Cout%d T%d" % (B, H, W, Ca, 2 * Cc, len(taps)))
-        ctx.cfg, ctx.conv_cfg, ctx.hw, ctx.flops = cfg, conv_cfg, (H, W), flops
+        ctx.cfg, ctx.conv_cfg, ctx.hw, ctx.flops, ctx.synced = cfg, conv_cfg, (H, W), flops, synced(cfg)
         ctx.skip_wgrad = _state["skip_wgrad"]
         ctx.weights = weights
         ctx.save_for_backward(actv, x, gamma, style, mean, rstd, amask)
@@ -873,7 +932,6 @@ class SpadeConvFn(torch.autograd.Function):
         Ca = actv.shape[3]
         st = L.stream()
         # ---- SPADE+Style backward (gamma kept alone: stride Cc)
-        racc = torch.empty(B * 5 * Cc + (B * 2 * Cc + 1) // 2, dtype=torch.float64, device=x.device)
         accumulate = sink is not None and sink.buf is not None
         dx = sink.buf if accumulate else torch.empty_like(x)      # at x's own resolution (see SpadeStyleFn.backward)
         last = True
@@ -886,9 +944,8 @@ class SpadeConvFn(torch.autograd.Function):
         dgb = torch.empty(B, H, W, 2 * Cc, dtype=BF16, device=x.device)
         dstyle = torch.empty_like(style) if style is not None else None
         chsum = torch.empty(3 * Cc, dtype=F32, device=x.device)
-        _timed_call("normb", 12.0 * B * H * W * Cc, "s2e_spade_style_bwd", L.ptr(dout), L.ptr(amask), L.ptr(x), L.ptr(gamma), L.ptr(style), L.ptr(mean),
-                    L.ptr(rstd), B, H * W, Cc, int(cfg.per_sample), cfg.act, L.ptr(racc), L.ptr(dx), int(accumulate), L.ptr(dgb),
-                    L.ptr(dstyle), L.ptr(chsum), W if up else 0, Cc, st, tag="bwd B%d HW%d C%d%s" % (B, H * W, Cc, " up" if up else ""))
+        _spade_style_bwd(ctx.synced, dout, amask, x, gamma, style, mean, rstd, B, H * W, Cc, int(cfg.per_sample), cfg.act, dx,
+                         accumulate, dgb, dstyle, chsum, W if up else 0, Cc, "bwd B%d HW%d C%d%s" % (B, H * W, Cc, " up" if up else ""))
         gx = None
         if last and ctx.needs_input_grad[1]:
             gx = dx

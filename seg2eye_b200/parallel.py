@@ -1,5 +1,7 @@
 """Data parallelism: one process per GPU, full replicas, batch sharded, per-rank BatchNorm statistics (what the
-reference's nn.DataParallel did, SURVEY.md 8(e)); the only collective is the gradient average.
+reference's nn.DataParallel did, SURVEY.md 8(e)); the only collective is the gradient average -- unless the SPADE layers
+share their statistics across ranks (`--norm_G spectralspadesyncbatch3x3`, ops.synced), which adds an all-gather per
+distinct SPADE input in forward and an all-reduce per SPADE layer in backward on the default group.
 
 GradReducer averages gradients with bucketed all-reduces that OVERLAP the backward pass: every parameter carries a
 post-accumulate-grad hook that copies its gradient into its bucket's flat fp32 buffer; when the last gradient of a
