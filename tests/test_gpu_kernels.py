@@ -263,7 +263,7 @@ def test_channel_padded_input_runs_d_first_layer_on_tensor_cores(S):
 
 def test_conv_tcgen05_large_k_many_tiles(S):
     L, ops = S
-    conv_case(S, L.IMPL_TC, 4, 512, 512, 20, 16, 3, 1, 1, 0, seed=3)         # K = 4608, persistent loop > 1 tile/CTA
+    conv_case(S, L.IMPL_TC, 4, 512, 512, 20, 16, 3, 1, 1, 0, seed=3)         # K = 4608, two N tiles, 20 work items: one per CTA
 
 
 # ------------------------------------------------------------------------------------------ spectral norm
@@ -1018,7 +1018,7 @@ HALO_CASES = [
     (1, 256, 128, 40, 32, 3, 1, 1, 1),     # four 64-channel blocks, fused LeakyReLU
     (2, 128, 64, 24, 16, 3, 1, 1, 0),
     (1, 64, 64, 37, 29, 3, 1, 1, 0),       # ragged: partial tiles right and bottom, odd tile count
-    (3, 128, 128, 40, 48, 3, 1, 1, 0),     # many tiles per CTA
+    (3, 128, 128, 40, 48, 3, 1, 1, 0),     # 54 halo tiles in 27 work items: one per CTA (test_gpu_conv_exact.py loops)
     (1, 64, 72, 16, 8, 3, 1, 1, 1),        # Cout not a multiple of 64
     (2, 64, 256, 24, 16, 3, 1, 1, 0),      # forward N = 256 (plain kernel), data gradient N = 64 (halo kernel)
 ]
