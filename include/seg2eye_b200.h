@@ -344,6 +344,18 @@ int s2e_adam_step(float* p, const float* g, float* m, float* v, long long n, con
 int s2e_adam_multi(int n_tensors, float* const* p, const float* const* g, float* const* m, float* const* v,
                    const long long* n, const float* state, float beta1, float beta2, float eps, float weight_decay,
                    void* stream);
+/* s2e_adam_multi plus an exponential moving average of the updated weights (--ema_decay, beyond the reference: the
+ * optimizer_G step of pix2pix_model.py:92-110 also advances netG_ema / netE_ema).  `ema` is a HOST array of n_tensors
+ * device pointers; after the Adam update of p, e <- fmaf(beta_t, e - p, p) in fp32 with
+ * beta_t = min(ema_decay, (1 + t) / (10 + t)) and t = state[0], the step count s2e_adam_prepare just advanced.
+ * 0 <= ema_decay < 1.  p, m, v come out bitwise equal to s2e_adam_multi's. */
+int s2e_adam_multi_ema(int n_tensors, float* const* p, const float* const* g, float* const* m, float* const* v,
+                       const long long* n, const float* state, float beta1, float beta2, float eps, float weight_decay,
+                       float* const* ema, float ema_decay, void* stream);
+/* dst[i] <- src[i] (nbytes[i] bytes, device memory, any dtype), one launch per 48 rows: the EMA nets take byte copies of
+ * the live nets' buffers (spectral-norm u/v, BatchNorm running statistics) after every optimizer_G step.  dst/src/nbytes
+ * are HOST arrays. */
+int s2e_copy_multi(int n_rows, void* const* dst, const void* const* src, const long long* nbytes, void* stream);
 int s2e_fill_f32(float* p, long long n, float value, void* stream);
 
 /* ------------------------------------------------------------------------------------------

@@ -61,6 +61,9 @@ _SIGS = {
     "s2e_spectral_power_iter_multi": [C.POINTER(SnJob), _I, _I, _I, _P],
     "s2e_pack_weight_multi": [C.POINTER(PackJob), _I, _P],
     "s2e_adam_multi": [_I, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_LL), _P, _F, _F, _F, _F, _P],
+    "s2e_adam_multi_ema": [_I, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_LL), _P, _F, _F, _F, _F,
+                           C.POINTER(_P), _F, _P],
+    "s2e_copy_multi": [_I, C.POINTER(_P), C.POINTER(_P), C.POINTER(_LL), _P],
     "s2e_sn_in_correction": [_P, _P, _P, _I, _I, _I, _F, _P, _P, _I, _P, _P, _P],
     "s2e_space_to_depth": [_P, _I, _I, _I, _I, _P, _P],
     "s2e_depth_to_space": [_P, _I, _I, _I, _I, _P, _P],

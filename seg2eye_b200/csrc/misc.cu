@@ -3,6 +3,8 @@
 #include <stdarg.h>
 #include <stdio.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 
 // ------------------------------------------------------------------------------------------ host state
@@ -964,6 +966,11 @@ struct AdamTable {
   long long n[ADAM_MAX_TENSORS];
   int blk0[ADAM_MAX_TENSORS];
 };
+// the EMA instantiation: e[k] is the moving average of p[k], decay the user's beta (the ramp is applied on the device)
+struct AdamEmaTable : AdamTable {
+  float* e[ADAM_MAX_TENSORS];
+  float decay;
+};
 __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, float b1, float b2, float eps, float wd,
                                          float step_size, float bc2_sqrt) {
   if (wd != 0.f) g = fmaf(wd, p, g);
@@ -972,8 +979,11 @@ __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, 
   const float denom = sqrtf(v) / bc2_sqrt + eps;
   p -= step_size * (m / denom);
 }
-__global__ void __launch_bounds__(256) adam_multi_kernel(const __grid_constant__ AdamTable t, const float* __restrict__ state,
-                                                         float b1, float b2, float eps, float wd) {
+// EMA = true: after the Adam update, e <- fmaf(beta_t, e - p, p) with the new p, where beta_t = min(decay, (1+t)/(10+t))
+// and t = state[0], the step count s2e_adam_prepare just advanced (so a CUDA-graph replay ramps correctly).
+template <bool EMA>
+__global__ void __launch_bounds__(256) adam_multi_kernel(const __grid_constant__ std::conditional_t<EMA, AdamEmaTable, AdamTable> t,
+                                                         const float* __restrict__ state, float b1, float b2, float eps, float wd) {
   int k = 0;
   while (k + 1 < t.nt && (int)blockIdx.x >= t.blk0[k + 1]) ++k;
   const long long off = (long long)(blockIdx.x - t.blk0[k]) * ADAM_CHUNK;
@@ -983,7 +993,13 @@ __global__ void __launch_bounds__(256) adam_multi_kernel(const __grid_constant__
   float* __restrict__ m = t.m[k] + off;
   float* __restrict__ v = t.v[k] + off;
   const float step_size = state[2], bc2_sqrt = state[3];
-  const bool aligned = ((((uintptr_t)p) | ((uintptr_t)g) | ((uintptr_t)m) | ((uintptr_t)v)) & 15) == 0;
+  float* __restrict__ ema = nullptr;
+  float bt = 0.f;
+  if constexpr (EMA) {
+    ema = t.e[k] + off;
+    bt = fminf(t.decay, (1.f + state[0]) / (10.f + state[0]));
+  }
+  const bool aligned = ((((uintptr_t)p) | ((uintptr_t)g) | ((uintptr_t)m) | ((uintptr_t)v) | ((uintptr_t)ema)) & 15) == 0;
   if (left >= ADAM_CHUNK && aligned) {
 #pragma unroll
     for (int i = 0; i < ADAM_CHUNK / (256 * 4); ++i) {
@@ -999,6 +1015,14 @@ __global__ void __launch_bounds__(256) adam_multi_kernel(const __grid_constant__
       *reinterpret_cast<float4*>(p + e) = pv;
       *reinterpret_cast<float4*>(m + e) = mv;
       *reinterpret_cast<float4*>(v + e) = vv;
+      if constexpr (EMA) {
+        float4 ev = *reinterpret_cast<float4*>(ema + e);
+        ev.x = fmaf(bt, ev.x - pv.x, pv.x);
+        ev.y = fmaf(bt, ev.y - pv.y, pv.y);
+        ev.z = fmaf(bt, ev.z - pv.z, pv.z);
+        ev.w = fmaf(bt, ev.w - pv.w, pv.w);
+        *reinterpret_cast<float4*>(ema + e) = ev;
+      }
     }
   } else {
     const int cnt = (int)(left < ADAM_CHUNK ? left : ADAM_CHUNK);
@@ -1008,8 +1032,36 @@ __global__ void __launch_bounds__(256) adam_multi_kernel(const __grid_constant__
       p[e] = pv;
       m[e] = mv;
       v[e] = vv;
+      if constexpr (EMA) ema[e] = fmaf(bt, ema[e] - pv, pv);
     }
   }
+}
+
+// Multi-tensor byte copy (the EMA nets' buffers): a block owns one COPY_CHUNK-byte chunk of one row of the table, moved
+// in 16-byte words when both ends are 16-byte aligned.
+constexpr int COPY_MAX_ROWS = 48;
+constexpr int COPY_CHUNK = 16384;
+struct CopyTable {
+  int nr;
+  void* dst[COPY_MAX_ROWS];
+  const void* src[COPY_MAX_ROWS];
+  long long nbytes[COPY_MAX_ROWS];
+  int blk0[COPY_MAX_ROWS];
+};
+__global__ void __launch_bounds__(256) copy_multi_kernel(const __grid_constant__ CopyTable t) {
+  int k = 0;
+  while (k + 1 < t.nr && (int)blockIdx.x >= t.blk0[k + 1]) ++k;
+  const long long off = (long long)(blockIdx.x - t.blk0[k]) * COPY_CHUNK;
+  const int cnt = (int)(t.nbytes[k] - off < COPY_CHUNK ? t.nbytes[k] - off : COPY_CHUNK);
+  unsigned char* d = (unsigned char*)t.dst[k] + off;
+  const unsigned char* s = (const unsigned char*)t.src[k] + off;
+  int head = 0;
+  if (((((uintptr_t)d) | ((uintptr_t)s)) & 15) == 0) {
+    head = cnt & ~15;
+    for (int i = threadIdx.x * 16; i < head; i += 256 * 16)
+      *reinterpret_cast<uint4*>(d + i) = *reinterpret_cast<const uint4*>(s + i);
+  }
+  for (int i = head + threadIdx.x; i < cnt; i += 256) d[i] = s[i];
 }
 
 PackGeom make_pack_geom(int Cout, int Cin, int kh, int kw, int stride, int pad, int Ctot = 0, int co_off = 0, int cin_pad = 0) {
@@ -1414,7 +1466,62 @@ int s2e_adam_multi(int n_tensors, float* const* p, const float* const* g, float*
       ++base;
     }
     if (t.nt == 0) break;
-    adam_multi_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(t, state, beta1, beta2, eps, weight_decay);
+    adam_multi_kernel<false><<<blocks, 256, 0, (cudaStream_t)stream>>>(t, state, beta1, beta2, eps, weight_decay);
+    S2E_LAUNCH_CHECK();
+  }
+  return S2E_OK;
+}
+int s2e_adam_multi_ema(int n_tensors, float* const* p, const float* const* g, float* const* m, float* const* v,
+                       const long long* n, const float* state, float beta1, float beta2, float eps, float weight_decay,
+                       float* const* ema, float ema_decay, void* stream) {
+  S2E_REQUIRE(n_tensors >= 0 && state && ema, "adam_multi_ema: bad arguments");
+  S2E_REQUIRE(ema_decay >= 0.f && ema_decay < 1.f, "adam_multi_ema: ema_decay %g is outside [0, 1)", (double)ema_decay);
+  for (int base = 0; base < n_tensors;) {
+    AdamEmaTable t;
+    t.nt = 0;
+    t.decay = ema_decay;
+    int blocks = 0;
+    while (base < n_tensors && t.nt < ADAM_MAX_TENSORS) {
+      if (n[base] > 0) {
+        S2E_REQUIRE(p[base] && g[base] && m[base] && v[base] && ema[base], "adam_multi_ema: tensor %d has a null pointer", base);
+        const int k = t.nt++;
+        t.p[k] = p[base];
+        t.g[k] = g[base];
+        t.m[k] = m[base];
+        t.v[k] = v[base];
+        t.e[k] = ema[base];
+        t.n[k] = n[base];
+        t.blk0[k] = blocks;
+        blocks += (int)ceil_div_ll(n[base], ADAM_CHUNK);
+      }
+      ++base;
+    }
+    if (t.nt == 0) break;
+    adam_multi_kernel<true><<<blocks, 256, 0, (cudaStream_t)stream>>>(t, state, beta1, beta2, eps, weight_decay);
+    S2E_LAUNCH_CHECK();
+  }
+  return S2E_OK;
+}
+int s2e_copy_multi(int n_rows, void* const* dst, const void* const* src, const long long* nbytes, void* stream) {
+  S2E_REQUIRE(n_rows >= 0, "copy_multi: bad row count");
+  for (int base = 0; base < n_rows;) {
+    CopyTable t;
+    t.nr = 0;
+    int blocks = 0;
+    while (base < n_rows && t.nr < COPY_MAX_ROWS) {
+      if (nbytes[base] > 0) {
+        S2E_REQUIRE(dst[base] && src[base], "copy_multi: row %d has a null pointer", base);
+        const int k = t.nr++;
+        t.dst[k] = dst[base];
+        t.src[k] = src[base];
+        t.nbytes[k] = nbytes[base];
+        t.blk0[k] = blocks;
+        blocks += (int)ceil_div_ll(nbytes[base], COPY_CHUNK);
+      }
+      ++base;
+    }
+    if (t.nr == 0) break;
+    copy_multi_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(t);
     S2E_LAUNCH_CHECK();
   }
   return S2E_OK;

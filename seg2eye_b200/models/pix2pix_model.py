@@ -8,6 +8,10 @@ the seg2eye_b200 kernels; what the reference computes and then throws away is no
   * torch.cat copies of [seg, image] (one layout kernel builds the D input), slices of the D features for the
     feature-matching loss (evaluated on the un-split [fake ; real] tensors).
 """
+import contextlib
+import copy
+import os
+
 import torch
 from torch import nn
 
@@ -24,15 +28,22 @@ class Pix2PixModel(torch.nn.Module):
     @staticmethod
     def modify_commandline_options(parser, is_train):
         networks.modify_commandline_options(parser, is_train)
+        parser.add_argument('--ema_decay', type=float, default=0.0,
+                            help='beyond the reference: keep an exponential moving average of the G and E weights with '
+                                 'this decay, 0 <= decay < 1 (0: off); inference uses it, saved as <epoch>_net_G_ema.pth')
         return parser
 
     def __init__(self, opt):
         super().__init__()
         self.opt = opt
+        self.ema_decay = optim.check_ema_decay(_opt(opt, 'ema_decay', 0.0))
         self.netG, self.netD, self.netE = self.initialize_networks(opt)
+        self.netG_ema = self.netE_ema = None
         self._last_d_out = None
         if not opt.isTrain:
             return
+        if self.ema_decay > 0:
+            self._initialize_ema(opt)
         if not _opt(opt, 'no_vgg_loss', True):
             raise ValueError('VGG loss does not exist in the reference either (networks.VGGLoss is undefined)')
         self.criterionGAN = networks.GANLoss(opt.gan_mode, opt=opt)
@@ -61,7 +72,8 @@ class Pix2PixModel(torch.nn.Module):
         return next(self.netG.parameters()).device
 
     def save(self, epoch):
-        for net, tag in ((self.netG, 'G'), (self.netD, 'D'), (self.netE, 'E')):
+        self.sync_ema()
+        for net, tag in ((self.netG, 'G'), (self.netD, 'D'), (self.netE, 'E'), (self.netG_ema, 'G_ema'), (self.netE_ema, 'E_ema')):
             if net is not None:
                 util.save_network(net, tag, epoch, self.opt)
 
@@ -71,12 +83,75 @@ class Pix2PixModel(torch.nn.Module):
         # --netG spade: the original style-less SPADE generator (BASELINE config 5) has no style encoder
         netE = networks.define_E(opt) if _opt(opt, 'netG', 'spadestyle') != 'spade' else None
         if not opt.isTrain or opt.continue_train:
-            util.load_network(netG, 'G', opt.which_epoch, opt)
+            # a model trained with --ema_decay is tested with the averaged generator
+            util.load_network(netG, 'G_ema' if not opt.isTrain and self.ema_decay > 0 else 'G', opt.which_epoch, opt)
             if opt.isTrain:   # like the reference, test time keeps a freshly initialised style encoder
                 util.load_network(netD, 'D', opt.which_epoch, opt)
                 if netE is not None:
                     util.load_network(netE, 'E', opt.which_epoch, opt)
         return netG, netD, netE
+
+    # ------------------------------------------------------------------ exponential moving average (--ema_decay)
+    def _initialize_ema(self, opt):
+        """netG_ema / netE_ema: frozen copies of netG / netE (or, on --continue_train, the saved averages when they exist)
+        that optimizer_G's Adam launch advances.  Their bf16 packed copies are refreshed by the first forward that reads
+        them after a G step (optim.Adam.ema_written), not by the training step (ops.pack_on_use)."""
+        def frozen_copy(net):
+            ema = copy.deepcopy(net, {id(opt): opt}).requires_grad_(False)
+            ops.pack_on_use(list(ema.parameters()))
+            return ema
+        self.netG_ema = frozen_copy(self.netG)
+        self.netE_ema = frozen_copy(self.netE) if self.netE is not None else None
+        if opt.continue_train:
+            for _, ema, tag in self._ema_pairs():
+                if os.path.exists(os.path.join(opt.checkpoints_dir, opt.name, '%s_net_%s_ema.pth' % (opt.which_epoch, tag))):
+                    util.load_network(ema, tag + '_ema', opt.which_epoch, opt)
+        self._ema_stale = False
+        for live, _, _ in self._ema_pairs():     # weights loaded into G / E from now on restart their averages
+            live.register_load_state_dict_post_hook(self._live_weights_replaced)
+
+    def _live_weights_replaced(self, module, incompatible_keys):
+        self._ema_stale = True
+
+    def _ema_pairs(self):
+        if self.netG_ema is None:
+            return []
+        return [(live, ema, tag) for live, ema, tag in ((self.netG, self.netG_ema, 'G'), (self.netE, self.netE_ema, 'E'))
+                if ema is not None]
+
+    @torch.no_grad()
+    def reset_ema(self):
+        """netG_ema / netE_ema <- netG / netE (parameters and buffers), in place: captured CUDA graphs keep their pointers."""
+        for live, ema, _ in self._ema_pairs():
+            for a, b in zip(list(ema.parameters()) + list(ema.buffers()), list(live.parameters()) + list(live.buffers())):
+                a.copy_(b)
+        self._ema_stale = False
+
+    def sync_ema(self):
+        """Restart the averages from the live nets if weights were loaded into G / E since (load_state_dict)."""
+        if self.netG_ema is not None and self._ema_stale:
+            self.reset_ema()
+
+    def ema_targets(self):
+        """optim.Adam's EMA arguments for the G+E optimizer: {parameter: average} and (EMA buffer, live buffer) pairs."""
+        pairs = self._ema_pairs()
+        ema = {p: e for live, em, _ in pairs for p, e in zip(live.parameters(), em.parameters())}
+        bufs = [(e, b) for live, em, _ in pairs for b, e in zip(live.buffers(), em.buffers())]
+        return dict(ema=ema, ema_buffers=bufs, ema_decay=self.ema_decay) if pairs else {}
+
+    @contextlib.contextmanager
+    def _inference_nets(self):
+        """The inference modes run netG_ema / netE_ema, when they exist, in place of netG / netE."""
+        if self.netG_ema is None:
+            yield
+            return
+        self.sync_ema()
+        live = self.netG, self.netE
+        self.netG, self.netE = self.netG_ema, self.netE_ema
+        try:
+            yield
+        finally:
+            self.netG, self.netE = live
 
     def create_optimizers(self, opt):
         """Adam over G+E and over D; TTUR (default) = betas (0, 0.9), lr/2 for G, lr*2 for D."""
@@ -87,7 +162,7 @@ class Pix2PixModel(torch.nn.Module):
         wd = _opt(opt, 'weight_decay', 0.0)
         g_params = list(self.netG.parameters()) + (list(self.netE.parameters()) if self.netE is not None else [])
         d_params = list(self.netD.parameters()) if opt.isTrain else []
-        return (optim.Adam(g_params, lr=g_lr, betas=betas, weight_decay=wd),
+        return (optim.Adam(g_params, lr=g_lr, betas=betas, weight_decay=wd, **self.ema_targets()),
                 optim.Adam(d_params, lr=d_lr, betas=betas, weight_decay=wd))
 
     # ------------------------------------------------------------------ entry point
@@ -98,9 +173,10 @@ class Pix2PixModel(torch.nn.Module):
         if mode == 'discriminator':
             return self.compute_discriminator_loss(seg, style, target)
         if mode == 'encode_only':
-            return self.encode_w(style)[0]
+            with self._inference_nets():
+                return self.encode_w(style)[0]
         if mode == 'inference':
-            with torch.no_grad():
+            with torch.no_grad(), self._inference_nets():
                 if 'latent_style' in data:
                     fake = self.generate_fake_from_stylecode(seg, data['latent_style'].to(seg.device))
                 else:

@@ -201,6 +201,15 @@ def mark_updated(params):
         p_._s2e_ver = getattr(p_, "_s2e_ver", 0) + 1
 
 
+def pack_on_use(tensors):
+    """Leave the packed copies of these tensors out of repack_stale(): they are re-packed only when a forward reads them
+    after their versions changed (mark_updated(), copy_, load_state_dict).  For the EMA nets (--ema_decay), whose
+    weights every G step changes but only an inference with them reads: re-packing them in the training step would
+    double its re-pack traffic."""
+    for t in tensors:
+        t._s2e_pack_on_use = True
+
+
 def _pack_jobs(entry, weights):
     jobs = []
     if entry.im2col:       # weights = (weight,) or (weight, bias): the bias goes to column 63
@@ -238,13 +247,16 @@ def repack_pending():
 
 
 def repack_stale():
-    """Re-pack every registered copy whose master weights changed, in one launch per 40 tensors."""
+    """Re-pack every registered copy whose master weights changed (except those of pack_on_use tensors), in one launch
+    per 40 tensors."""
     _state["packed_epoch"] = _state["weights_epoch"]
     jobs, dead = [], []
     for key, e in _pack_cache.items():
         ws = e.weights()
         if ws is None:
             dead.append(key)
+            continue
+        if any(getattr(w, "_s2e_pack_on_use", False) for w in ws):
             continue
         ver = _master_version(ws)
         if ver != e.ver:

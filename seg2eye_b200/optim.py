@@ -7,10 +7,29 @@ from . import _lib as L
 from . import ops
 
 
+def check_ema_decay(beta):
+    beta = float(beta)
+    if not 0.0 <= beta < 1.0:
+        raise ValueError("ema_decay must be in [0, 1), got %r" % beta)
+    return beta
+
+
 class Adam(torch.optim.Optimizer):
-    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0):
+    """`ema` (optional): {parameter: tensor of the same shape} -- after every step each such parameter's moving average
+    advances, e <- fmaf(beta_t, e - p, p) with beta_t = min(ema_decay, (1 + t) / (10 + t)) at step count t, in the Adam
+    launch itself.  `ema_buffers`: (destination, source) tensor pairs byte-copied after every step, in one more launch.
+    Neither is part of the optimizer's state_dict.  The packed bf16 copies of the EMA tensors are not re-packed here
+    (ops.pack_on_use): ema_written() marks them stale, and the next forward that reads them re-packs them."""
+
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, ema=None, ema_buffers=(),
+                 ema_decay=0.0):
         defaults = dict(lr=lr, betas=(float(betas[0]), float(betas[1])), eps=eps, weight_decay=weight_decay)
         super().__init__(params, defaults)
+        self.ema, self.ema_buffers, self.ema_decay = ema, list(ema_buffers), check_ema_decay(ema_decay)
+        for p, e in (ema or {}).items():
+            assert e.shape == p.shape and e.dtype == torch.float32 and e.is_contiguous()
+        for d, s_ in self.ema_buffers:
+            assert d.dtype == s_.dtype and d.shape == s_.shape and d.is_contiguous() and s_.is_contiguous()
 
     def _dev_state(self, group):
         ps = [p for p in group['params'] if p.grad is not None]
@@ -32,8 +51,9 @@ class Adam(torch.optim.Optimizer):
 
     @torch.no_grad()
     def step(self, closure=None):
-        """One multi-tensor launch per 48 parameters, then one multi-tensor re-pack of the bf16 copies of the weights
-        that just changed (ops.repack_stale) -- both capturable in a CUDA graph."""
+        """One multi-tensor launch per 48 parameters (with the EMA update when `ema` is set, then the buffer copies), then
+        one multi-tensor re-pack of the bf16 copies of the weights that just changed (ops.repack_stale) -- all capturable
+        in a CUDA graph."""
         import ctypes as C
         s = L.stream()
         touched = []
@@ -54,8 +74,24 @@ class Adam(torch.optim.Optimizer):
                 rows.append((L.ptr(p), L.ptr(g), L.ptr(state['exp_avg']), L.ptr(state['exp_avg_sq']), p.numel(), g))
             n = len(rows)
             arr = lambda k: (C.c_void_p * n)(*[r[k] for r in rows])
-            L.call("s2e_adam_multi", n, arr(0), arr(1), arr(2), arr(3), (C.c_longlong * n)(*[r[4] for r in rows]),
-                   L.ptr(st), b1, b2, group['eps'], group['weight_decay'], s)
+            args = (n, arr(0), arr(1), arr(2), arr(3), (C.c_longlong * n)(*[r[4] for r in rows]),
+                    L.ptr(st), b1, b2, group['eps'], group['weight_decay'])
+            if self.ema:
+                L.call("s2e_adam_multi_ema", *args, (C.c_void_p * n)(*[L.ptr(self.ema[p]) for p in ps]), self.ema_decay, s)
+            else:
+                L.call("s2e_adam_multi", *args, s)
             touched += ps
+        if self.ema_buffers:
+            n = len(self.ema_buffers)
+            L.call("s2e_copy_multi", n, (C.c_void_p * n)(*[L.ptr(d) for d, _ in self.ema_buffers]),
+                   (C.c_void_p * n)(*[L.ptr(s_) for _, s_ in self.ema_buffers]),
+                   (C.c_longlong * n)(*[s_.numel() * s_.element_size() for _, s_ in self.ema_buffers]), s)
+        self.ema_written()
         ops.mark_updated(touched)
         ops.repack_stale()
+
+    def ema_written(self):
+        """The kernel wrote the averages through raw pointers: bump their versions so that their packed copies re-pack at
+        their next use.  Also called after every replay of a captured step, which runs no Python."""
+        if self.ema:
+            ops.mark_updated(self.ema.values())

@@ -27,8 +27,8 @@ class Pix2PixTrainer():
         m = self.pix2pix_model
         if self.world > 1:
             # every replica must start from the same weights AND the same spectral-norm u/v / BatchNorm buffers (both are
-            # randomly initialised per process)
-            for net in (m.netG, m.netD, m.netE):
+            # randomly initialised per process); the EMA nets are rank 0's copies of its G / E or its loaded averages
+            for net in (m.netG, m.netD, m.netE, m.netG_ema, m.netE_ema):
                 if net is not None:
                     parallel.broadcast_module(net, 0)
             from .. import ops
@@ -108,7 +108,9 @@ class Pix2PixTrainer():
                         'target': example_data['target'].float().to(dev).clone()}
         if 'style_image' in example_data:
             self._static['style_image'] = example_data['style_image'].float().to(dev).clone()
-        tensors = [t for net in (m.netG, m.netD, m.netE) if net is not None for t in list(net.parameters()) + list(net.buffers())]
+        m.sync_ema()
+        tensors = [t for net in (m.netG, m.netD, m.netE, m.netG_ema, m.netE_ema) if net is not None
+                   for t in list(net.parameters()) + list(net.buffers())]
         opts = (self.optimizer_G, self.optimizer_D)
         if multi:     # the capture set-up below runs on a side stream: no all-reduce launches from inside backward there
             self.reducer_G.remove_hooks()
@@ -185,8 +187,9 @@ class Pix2PixTrainer():
         self._graphs = True
 
     def reset_optimizers(self):
-        """Both optimizers as freshly constructed: zero Adam moments and step counts, written in place so that captured
-        CUDA graphs keep reading the same tensors."""
+        """Both optimizers as freshly constructed: zero Adam moments and step counts, and the EMA nets copies of G / E,
+        written in place so that captured CUDA graphs keep reading the same tensors."""
+        self.pix2pix_model.reset_ema()
         for o in (self.optimizer_G, self.optimizer_D):
             for st in o.state.values():
                 st['exp_avg'].zero_()
@@ -224,6 +227,8 @@ class Pix2PixTrainer():
         if g_opt is not None:
             (self.reducer_G if which == 'G' else self.reducer_D).allreduce_flat()
             g_opt.replay()
+        if which == 'G':
+            self.optimizer_G.ema_written()
         for k, vals in log.items():
             for v in vals:
                 self.pix2pix_model.add_to_loss_log(k, v.clone())
@@ -231,6 +236,7 @@ class Pix2PixTrainer():
 
     # ------------------------------------------------------------------ reference API
     def run_generator_one_step(self, data):
+        self.pix2pix_model.sync_ema()
         if self._graphs:
             self.g_losses, self.generated = self._replay('G', data)
         else:
