@@ -308,6 +308,49 @@ int s2e_tanh_bwd(const float* dy, const float* y, long long n, void* dx_bf16, vo
 /* gradient of the fake image w.r.t. the D input channel nc (first B samples) -> fp32 (B,1,H,W) */
 int s2e_d_input_grad(const void* dxin, int B, int nc, int H, int W, int Cpad, float* dfake, void* stream);
 
+/* Differentiable augmentation of the D input (--diff_augment, beyond the reference; DiffAugment, Zhao et al., NeurIPS
+ * 2020: rand_brightness, rand_saturation, rand_contrast, rand_translation, rand_cutout, applied in that order).
+ *
+ * Parameters.  s2e_diffaug_draw writes one record of S2E_DIFFAUG_RECORD fp32 values per sample b < B,
+ *     (u0, u1, tx, ty, ox, oy),
+ * from Philox4x32-10 with key = (seed lo, seed hi) and counter = (n, ctr lo, ctr hi, blk), where state[0] = seed,
+ * state[1] = ctr (both int64, device memory) and n = index_offset + b (the sample's global index, < 2^32).  Block
+ * blk = 0 gives the words (r0, r1, r2, r3), block 1 gives (r4, r5, -, -).  A word r maps to
+ *     a float in [0, 1):        (r >> 8) * 2^-24
+ *     an integer in [0, n):     (r * n) >> 32        (64-bit product)
+ * and   u0 = float(r0), u1 = float(r1),
+ *       tx = int(r2, 2 sx + 1) - sx,  ty = int(r3, 2 sy + 1) - sy,   sx = (H + 4) / 8, sy = (W + 4) / 8  (= int(H/8 + 0.5)),
+ *       ox = int(r4, H + 1 - cx % 2), oy = int(r5, W + 1 - cy % 2),  cx = (H + 1) / 2, cy = (W + 1) / 2  (= int(H/2 + 0.5)).
+ * All six are drawn whatever the policy, so an op's parameters never depend on which other ops are on.  One launch
+ * (one block); it reads ctr on the device and then sets state[1] = ctr + 1, so every replay of a captured CUDA graph
+ * draws new parameters.
+ *
+ * Ops, per sample, on the H x W map (policy = OR of the S2E_DIFFAUG_* bits; row b of [fake ; real] and row B + b use
+ * record b):
+ *   COLOR (image channel only):  x'' = (x' - mean(x')) (u1 + 0.5) + mean(x'),  x' = x + (u0 - 0.5), the mean over the
+ *       H x W pixels of that image (s2e_diffaug_means: fp32 values, fp64 sums).  Saturation is the identity on one
+ *       channel and is not drawn.
+ *   TRANSLATION (every channel):  out[i, j] = in[i + tx, j + ty], 0 where that index is outside the map.
+ *   CUTOUT (every channel):  out[i, j] = 0 for ox - cx/2 <= i < ox - cx/2 + cx and oy - cy/2 <= j < oy - cy/2 + cy. */
+#define S2E_DIFFAUG_COLOR 1
+#define S2E_DIFFAUG_TRANSLATION 2
+#define S2E_DIFFAUG_CUTOUT 4
+#define S2E_DIFFAUG_ALL 7
+#define S2E_DIFFAUG_RECORD 6
+int s2e_diffaug_draw(int64_t* state, int B, long long index_offset, int H, int W, float* params_out, void* stream);
+/* means_out[b] = mean(fake[b]), means_out[B + b] = mean(real[b]); fake, real fp32 (B,1,H,W) */
+int s2e_diffaug_means(const float* fake, const float* real, int B, int H, int W, float* means_out, void* stream);
+/* s2e_make_d_input with the policy applied while gathering (colour in fp32 on the image value, one rounding to bf16);
+ * channels nc + 1 .. Cpad - 1 stay zero.  means: s2e_diffaug_means's output, needed with COLOR only. */
+int s2e_make_d_input_aug(const float* seg_nchw, const float* fake, const float* real, int B, int nc, int H, int W,
+                         int Cpad, const float* params, const float* means, int policy, void* out, void* stream);
+/* adjoint of s2e_make_d_input_aug for the fake image: g'[i, j] = dxin[b, i - tx, j - ty, nc] (0 where that output pixel
+ * does not exist or is cut out), then with COLOR dfake = c g' + (1 - c) mean(g'), c = u1 + 0.5 (brightness passes the
+ * gradient unchanged).  scratch: B doubles (the per-sample sums of g'), needed with COLOR only; two launches with COLOR,
+ * one without. */
+int s2e_d_input_grad_aug(const void* dxin, int B, int nc, int H, int W, int Cpad, const float* params, int policy,
+                         double* scratch, float* dfake, void* stream);
+
 /* small fp32 linear layers: y = act(x W^T + b).  FC 16->2C (normalization.py:134-141), fc_mu/fc_var
  * (encoder.py:68-71).  in_nhwc_hw > 0: x is bf16 NHWC [M, hw, K/hw] flattened in NCHW order with LeakyReLU(0.2)
  * applied to the input first (encoder.py:64-67). */

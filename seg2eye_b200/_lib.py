@@ -13,6 +13,8 @@ MAX_TAPS = 16
 ACT_NONE, ACT_LRELU, ACT_RELU = 0, 1, 2
 IMPL_TC, IMPL_SIMT = 0, 1
 RED_SUM, RED_HINGE_REAL, RED_HINGE_FAKE, RED_L1, RED_L2, RED_LS, RED_BCE = 0, 1, 2, 3, 4, 5, 6
+DIFFAUG_COLOR, DIFFAUG_TRANSLATION, DIFFAUG_CUTOUT = 1, 2, 4
+DIFFAUG_RECORD = 6
 
 
 class ConvDesc(C.Structure):
@@ -89,6 +91,10 @@ _SIGS = {
     "s2e_bilinear_bwd": [_P, _I, _I, _I, _I, _I, _P, _P],
     "s2e_make_d_input": [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P],
     "s2e_d_input_grad": [_P, _I, _I, _I, _I, _I, _P, _P],
+    "s2e_diffaug_draw": [_P, _I, _LL, _I, _I, _P, _P],
+    "s2e_diffaug_means": [_P, _P, _I, _I, _I, _P, _P],
+    "s2e_make_d_input_aug": [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P],
+    "s2e_d_input_grad_aug": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P],
     "s2e_tanh_fwd": [_P, _LL, _P, _P],
     "s2e_tanh_bwd": [_P, _P, _LL, _P, _P],
     "s2e_linear_fwd": [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P],

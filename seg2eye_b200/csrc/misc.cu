@@ -740,6 +740,172 @@ __global__ void d_input_grad_kernel(const bf16* __restrict__ dxin, int nc, int C
   GRID_STRIDE(i, n) dfake[i] = __bfloat162float(dxin[i * Cpad + nc]);
 }
 
+// ------------------------------------------------------------------------------------------ differentiable augmentation
+// DiffAugment (Zhao et al., NeurIPS 2020) of the D input; the formulas and the record layout are in the header.
+// Philox4x32-10 (Salmon et al., SC'11), the generator of curand / Random123: 10 rounds, the key bumped between rounds.
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r) {
+      k.x += 0x9E3779B9u;
+      k.y += 0xBB67AE85u;
+    }
+    const unsigned lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
+    const unsigned lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+  }
+  return c;
+}
+__device__ __forceinline__ float da_unit(unsigned r) { return (float)(r >> 8) * (1.f / 16777216.f); }
+__device__ __forceinline__ int da_below(unsigned r, int n) { return (int)(((unsigned long long)r * (unsigned)n) >> 32); }
+
+// one block: thread t writes the records of samples t, t + 256, ... from the counter it read, then thread 0 advances it
+__global__ void __launch_bounds__(256) diffaug_draw_kernel(long long* state, int B, long long index_offset, int H, int W,
+                                                           float* __restrict__ rec) {
+  const unsigned long long seed = (unsigned long long)state[0], ctr = (unsigned long long)state[1];
+  const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
+  const int sx = (H + 4) / 8, sy = (W + 4) / 8;    // int(H / 8 + 0.5)
+  const int cx = (H + 1) / 2, cy = (W + 1) / 2;    // int(H / 2 + 0.5)
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    const unsigned idx = (unsigned)(index_offset + b);
+    const uint4 r0 = philox4x32_10(make_uint4(idx, (unsigned)ctr, (unsigned)(ctr >> 32), 0u), key);
+    const uint4 r1 = philox4x32_10(make_uint4(idx, (unsigned)ctr, (unsigned)(ctr >> 32), 1u), key);
+    float* o = rec + (long long)b * S2E_DIFFAUG_RECORD;
+    o[0] = da_unit(r0.x);
+    o[1] = da_unit(r0.y);
+    o[2] = (float)(da_below(r0.z, 2 * sx + 1) - sx);
+    o[3] = (float)(da_below(r0.w, 2 * sy + 1) - sy);
+    o[4] = (float)da_below(r1.x, H + 1 - cx % 2);
+    o[5] = (float)da_below(r1.y, W + 1 - cy % 2);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) state[1] = (long long)(ctr + 1);
+}
+
+__device__ __forceinline__ double block_sum_f64(double v) {
+  __shared__ double sh[32];
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+  if (l == 0) sh[w] = v;
+  __syncthreads();
+  const int nw = (blockDim.x + 31) >> 5;
+  v = (threadIdx.x < nw) ? sh[threadIdx.x] : 0.0;
+  if (w == 0)
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;  // valid in thread 0
+}
+
+// per-image means for contrast: block b2 reduces fake[b2] (b2 < B) or real[b2 - B] in fp64
+__global__ void __launch_bounds__(1024) diffaug_means_kernel(const float* __restrict__ fake, const float* __restrict__ real, int B,
+                                                             long long HW, float* __restrict__ means) {
+  const int b2 = blockIdx.x;
+  const float* x = (b2 < B ? fake : real) + (long long)(b2 % B) * HW;
+  double s0 = 0.0, s1 = 0.0;
+  long long i = threadIdx.x;
+  for (; i + blockDim.x < HW; i += 2 * blockDim.x) {
+    s0 += (double)x[i];
+    s1 += (double)x[i + blockDim.x];
+  }
+  if (i < HW) s0 += (double)x[i];
+  const double s = block_sum_f64(s0 + s1);
+  if (threadIdx.x == 0) means[b2] = (float)(s / (double)HW);
+}
+
+// is output pixel (i, j) of a sample with record r outside its cutout rectangle?
+__device__ __forceinline__ bool da_not_cut(int i, int j, int H, int W, const float* r, int policy) {
+  if (policy & S2E_DIFFAUG_CUTOUT) {
+    const int cx = (H + 1) / 2, cy = (W + 1) / 2;
+    const int x0 = (int)r[4] - cx / 2, y0 = (int)r[5] - cy / 2;
+    if (i >= x0 && i < x0 + cx && j >= y0 && j < y0 + cy) return false;
+  }
+  return true;
+}
+
+// make_d_input_kernel with the augmentation applied while gathering: one thread per output pixel of the (2B, H, W) batch
+template <bool COLOR>
+__global__ void make_d_input_aug_kernel(const float* __restrict__ seg, const float* __restrict__ fake, const float* __restrict__ real,
+                                        int B, int nc, int H, int W, int Cpad, long long npix, const float* __restrict__ rec,
+                                        const float* __restrict__ means, int policy, bf16* __restrict__ out) {
+  const long long HW = (long long)H * W;
+  GRID_STRIDE(p, npix) {
+    const long long hw = p % HW;
+    const int b2 = (int)(p / HW);
+    const int b = b2 % B;
+    const float* r = rec + (long long)b * S2E_DIFFAUG_RECORD;
+    const int i = (int)(hw / W), j = (int)(hw % W);
+    int si = i, sj = j;
+    if (policy & S2E_DIFFAUG_TRANSLATION) {
+      si += (int)__ldg(r + 2);
+      sj += (int)__ldg(r + 3);
+    }
+    const bool keep = si >= 0 && si < H && sj >= 0 && sj < W && da_not_cut(i, j, H, W, r, policy);
+    const long long shw = keep ? (long long)si * W + sj : 0;
+    const float* sp = seg + (long long)b * nc * HW + shw;
+    float img = 0.f;
+    if (keep) {
+      img = (b2 < B ? fake : real)[(long long)b * HW + shw];
+      if (COLOR) {   // brightness, then contrast around the brightened image's mean (saturation: identity on 1 channel)
+        const float br = __ldg(r) - 0.5f, ct = __ldg(r + 1) + 0.5f;
+        const float mb = __ldg(means + b2) + br;
+        img = (img + br - mb) * ct + mb;
+      }
+    }
+    bf16* o = out + p * Cpad;
+    if ((Cpad & 7) == 0) {
+      for (int c0 = 0; c0 < Cpad; c0 += 8) {
+        float v[8];
+#pragma unroll
+        for (int jj = 0; jj < 8; ++jj) {
+          const int c = c0 + jj;
+          v[jj] = c < nc ? (keep ? sp[(long long)c * HW] : 0.f) : (c == nc ? img : 0.f);
+        }
+        st_stream8(o + c0, pack8(v));
+      }
+    } else {
+      for (int c = 0; c < Cpad; ++c) o[c] = __float2bfloat16(c < nc ? (keep ? sp[(long long)c * HW] : 0.f) : (c == nc ? img : 0.f));
+    }
+  }
+}
+
+// g'(b, i, j): the gradient of output channel nc at the pixel that read source (i, j), 0 if none did
+__device__ __forceinline__ float da_grad_gather(const bf16* __restrict__ dxin, int nc, int Cpad, int H, int W, int b, int i, int j,
+                                                const float* r, int policy) {
+  int oi = i, oj = j;
+  if (policy & S2E_DIFFAUG_TRANSLATION) {
+    oi -= (int)__ldg(r + 2);
+    oj -= (int)__ldg(r + 3);
+  }
+  if (oi < 0 || oi >= H || oj < 0 || oj >= W || !da_not_cut(oi, oj, H, W, r, policy)) return 0.f;
+  return __bfloat162float(dxin[(((long long)b * H + oi) * W + oj) * Cpad + nc]);
+}
+// contrast's adjoint needs sum(g') per sample: block b reduces it in fp64
+__global__ void __launch_bounds__(1024) d_input_grad_aug_sum_kernel(const bf16* __restrict__ dxin, int nc, int Cpad, int H, int W,
+                                                                    const float* __restrict__ rec, int policy, double* __restrict__ sums) {
+  const int b = blockIdx.x;
+  const float* r = rec + (long long)b * S2E_DIFFAUG_RECORD;
+  double s = 0.0;
+  for (long long hw = threadIdx.x; hw < (long long)H * W; hw += blockDim.x)
+    s += (double)da_grad_gather(dxin, nc, Cpad, H, W, b, (int)(hw / W), (int)(hw % W), r, policy);
+  s = block_sum_f64(s);
+  if (threadIdx.x == 0) sums[b] = s;
+}
+template <bool COLOR>
+__global__ void d_input_grad_aug_kernel(const bf16* __restrict__ dxin, int B, int nc, int Cpad, int H, int W, const float* __restrict__ rec,
+                                        int policy, const double* __restrict__ sums, float* __restrict__ dfake) {
+  const long long HW = (long long)H * W;
+  GRID_STRIDE(p, (long long)B * HW) {
+    const int b = (int)(p / HW);
+    const long long hw = p % HW;
+    const float* r = rec + (long long)b * S2E_DIFFAUG_RECORD;
+    float g = da_grad_gather(dxin, nc, Cpad, H, W, b, (int)(hw / W), (int)(hw % W), r, policy);
+    if (COLOR) {   // dfake = c g' + (1 - c) mean(g')
+      const float ct = __ldg(r + 1) + 0.5f;
+      g = fmaf(ct, g, (1.f - ct) * (float)(__ldg(sums + b) / (double)HW));
+    }
+    dfake[p] = g;
+  }
+}
+
 // ------------------------------------------------------------------------------------------ elementwise
 __global__ void add_kernel(const bf16* __restrict__ a, const bf16* __restrict__ b, long long nvec, long long n, bf16* __restrict__ y) {
   GRID_STRIDE(i, nvec) {
@@ -1368,6 +1534,50 @@ int s2e_d_input_grad(const void* dxin, int B, int nc, int H, int W, int Cpad, fl
   const long long n = (long long)B * H * W;
   if (!n) return S2E_OK;
   d_input_grad_kernel<<<grid1d(n), NT, 0, (cudaStream_t)stream>>>((const bf16*)dxin, nc, Cpad, n, dfake);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_diffaug_draw(int64_t* state, int B, long long index_offset, int H, int W, float* params_out, void* stream) {
+  S2E_REQUIRE(state && B >= 0 && H > 0 && W > 0 && index_offset >= 0, "diffaug_draw: bad arguments");
+  S2E_REQUIRE(index_offset + B <= (1LL << 32), "diffaug_draw: sample indices must fit in 32 bits");
+  S2E_REQUIRE(B == 0 || params_out, "diffaug_draw: params_out is null");
+  diffaug_draw_kernel<<<1, 256, 0, (cudaStream_t)stream>>>((long long*)state, B, index_offset, H, W, params_out);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_diffaug_means(const float* fake, const float* real, int B, int H, int W, float* means_out, void* stream) {
+  S2E_REQUIRE(B >= 0 && H > 0 && W > 0, "diffaug_means: bad arguments");
+  if (!B) return S2E_OK;
+  diffaug_means_kernel<<<2 * B, 1024, 0, (cudaStream_t)stream>>>(fake, real, B, (long long)H * W, means_out);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_make_d_input_aug(const float* seg, const float* fake, const float* real, int B, int nc, int H, int W, int Cpad,
+                         const float* params, const float* means, int policy, void* out, void* stream) {
+  S2E_REQUIRE(Cpad > nc, "make_d_input_aug: Cpad must exceed nc");
+  S2E_REQUIRE((policy & ~S2E_DIFFAUG_ALL) == 0, "make_d_input_aug: unknown policy bits %#x", policy);
+  S2E_REQUIRE(params && (means || !(policy & S2E_DIFFAUG_COLOR)), "make_d_input_aug: params / means missing");
+  const long long npix = 2LL * B * H * W;
+  if (!npix) return S2E_OK;
+  auto k = (policy & S2E_DIFFAUG_COLOR) ? make_d_input_aug_kernel<true> : make_d_input_aug_kernel<false>;
+  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_d_input_grad_aug(const void* dxin, int B, int nc, int H, int W, int Cpad, const float* params, int policy,
+                         double* scratch, float* dfake, void* stream) {
+  S2E_REQUIRE((policy & ~S2E_DIFFAUG_ALL) == 0, "d_input_grad_aug: unknown policy bits %#x", policy);
+  S2E_REQUIRE(params && (scratch || !(policy & S2E_DIFFAUG_COLOR)), "d_input_grad_aug: params / scratch missing");
+  const long long n = (long long)B * H * W;
+  if (!n) return S2E_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (policy & S2E_DIFFAUG_COLOR) {
+    d_input_grad_aug_sum_kernel<<<B, 1024, 0, st>>>((const bf16*)dxin, nc, Cpad, H, W, params, policy, scratch);
+    S2E_LAUNCH_CHECK();
+    d_input_grad_aug_kernel<true><<<grid1d(n), NT, 0, st>>>((const bf16*)dxin, B, nc, Cpad, H, W, params, policy, scratch, dfake);
+  } else {
+    d_input_grad_aug_kernel<false><<<grid1d(n), NT, 0, st>>>((const bf16*)dxin, B, nc, Cpad, H, W, params, policy, nullptr, dfake);
+  }
   S2E_LAUNCH_CHECK();
   return S2E_OK;
 }

@@ -8,6 +8,7 @@ the seg2eye_b200 kernels; what the reference computes and then throws away is no
   * torch.cat copies of [seg, image] (one layout kernel builds the D input), slices of the D features for the
     feature-matching loss (evaluated on the un-split [fake ; real] tensors).
 """
+import argparse
 import contextlib
 import copy
 import os
@@ -16,12 +17,20 @@ import torch
 from torch import nn
 
 from .. import _lib as L
-from .. import ops, optim, util
+from .. import ops, optim, parallel, util
 from . import networks
 
 
 def _opt(opt, name, default=0):
     return getattr(opt, name, default)
+
+
+def _diff_augment_arg(value):
+    """--diff_augment: unknown ops are rejected while parsing; the value comes back in canonical order."""
+    try:
+        return ','.join(ops.parse_diff_augment(value)[0])
+    except ValueError as e:
+        raise argparse.ArgumentTypeError(str(e))
 
 
 class Pix2PixModel(torch.nn.Module):
@@ -31,17 +40,28 @@ class Pix2PixModel(torch.nn.Module):
         parser.add_argument('--ema_decay', type=float, default=0.0,
                             help='beyond the reference: keep an exponential moving average of the G and E weights with '
                                  'this decay, 0 <= decay < 1 (0: off); inference uses it, saved as <epoch>_net_G_ema.pth')
+        parser.add_argument('--diff_augment', type=_diff_augment_arg, default='',
+                            help='beyond the reference: differentiable augmentation of everything D sees in training '
+                                 '(DiffAugment), a comma-separated subset of color,translation,cutout (always applied in '
+                                 'that order; empty: off)')
         return parser
 
     def __init__(self, opt):
         super().__init__()
         self.opt = opt
         self.ema_decay = optim.check_ema_decay(_opt(opt, 'ema_decay', 0.0))
+        self.diffaug_ops, self.diffaug_policy = ops.parse_diff_augment(_opt(opt, 'diff_augment', ''))
         self.netG, self.netD, self.netE = self.initialize_networks(opt)
         self.netG_ema = self.netE_ema = None
+        self.diffaug_state = None
         self._last_d_out = None
         if not opt.isTrain:
             return
+        if self.diffaug_policy:
+            # int64 [seed, draw counter] on the device: s2e_diffaug_draw reads and advances the counter there, so replays
+            # of a captured step draw new parameters.  Held here, not by netD, whose state_dict keeps the reference's keys.
+            seed = int(torch.randint(-2 ** 63, 2 ** 63 - 1, (), dtype=torch.int64))
+            self.diffaug_state = torch.tensor([seed, 0], dtype=torch.int64, device=self.device())
         if self.ema_decay > 0:
             self._initialize_ema(opt)
         if not _opt(opt, 'no_vgg_loss', True):
@@ -328,9 +348,18 @@ class Pix2PixModel(torch.nn.Module):
     # ------------------------------------------------------------------ discriminator call
     def discriminate(self, input_semantics, fake_image, real_image):
         """cat([seg,fake],1) / cat([seg,real],1) / cat(.,0) of the reference as ONE layout kernel; channels are
-        zero-padded to 16 so that D's first 4x4-s2 convolution is tensor-core shaped after space-to-depth."""
+        zero-padded to 16 so that D's first 4x4-s2 convolution is tensor-core shaped after space-to-depth.
+        With --diff_augment, in training, the layout kernel's augmented twin builds it: one parameter record per sample
+        pair (fake b and real b alike, so the feature-matching loss still compares aligned images), drawn for the
+        sample's global index rank * B + b."""
         # (5 -> 16 channels for the 4-class OpenEDS maps; in general the next multiple of 16)
-        both = ops.MakeDInputFn.apply(input_semantics, fake_image, real_image, -(-(input_semantics.shape[1] + 1) // 16) * 16)
+        cpad = -(-(input_semantics.shape[1] + 1) // 16) * 16
+        if self.diffaug_policy and self.training:
+            B, _, H, W = input_semantics.shape
+            params = ops.diffaug_draw(self.diffaug_state, B, parallel.rank() * B, H, W)
+            both = ops.MakeDInputAugFn.apply(input_semantics, fake_image, real_image, cpad, params, self.diffaug_policy)
+        else:
+            both = ops.MakeDInputFn.apply(input_semantics, fake_image, real_image, cpad)
         out = self.netD.forward_nhwc(both)
         self._last_d_out = out
         return self.divide_pred(out)

@@ -1310,6 +1310,68 @@ class MakeDInputFn(torch.autograd.Function):
         return None, dfake, None, None
 
 
+DIFFAUG_OPS = (("color", L.DIFFAUG_COLOR), ("translation", L.DIFFAUG_TRANSLATION), ("cutout", L.DIFFAUG_CUTOUT))
+
+
+def parse_diff_augment(policy):
+    """'cutout,color' -> ('color', 'cutout'), the bits of the C ABI: the ops always run in DiffAugment's order color ->
+    translation -> cutout, whatever the order of the string.  '' -> ((), 0)."""
+    names = [s.strip() for s in (policy or '').split(',') if s.strip()]
+    known = dict(DIFFAUG_OPS)
+    bad = [n for n in names if n not in known]
+    if bad:
+        raise ValueError("--diff_augment: unknown op(s) %s (choose from %s)" % (bad, ", ".join(known)))
+    ops_ = tuple(n for n, _ in DIFFAUG_OPS if n in names)
+    return ops_, sum(known[n] for n in ops_)
+
+
+def diffaug_draw(state, B, index_offset, H, W):
+    """[B, 6] fp32 parameter records (u0, u1, tx, ty, ox, oy) of samples index_offset .. index_offset + B - 1 for an H x W
+    map, drawn at the counter in `state` (int64 [seed, counter] on the device), which the launch advances by one."""
+    assert state.dtype == torch.int64 and state.numel() == 2 and state.is_contiguous()
+    rec = torch.empty(B, L.DIFFAUG_RECORD, dtype=F32, device=state.device)
+    L.call("s2e_diffaug_draw", L.ptr(state), B, index_offset, H, W, L.ptr(rec), L.stream())
+    return rec
+
+
+class MakeDInputAugFn(torch.autograd.Function):
+    """MakeDInputFn with differentiable augmentation (--diff_augment): rows b and B + b use record b of `params`
+    (ops.diffaug_draw); colour touches the image channel, translation and cutout every channel."""
+
+    @staticmethod
+    def forward(ctx, seg, fake, real, cpad, params, policy):
+        seg, fake, real = _c(seg.float()), _c(fake.float()), _c(real.float())
+        B, nc, H, W = seg.shape
+        assert fake.shape == (B, 1, H, W) and real.shape == (B, 1, H, W), (fake.shape, real.shape, seg.shape)
+        assert params.shape == (B, L.DIFFAUG_RECORD) and params.dtype == F32 and params.is_contiguous()
+        cpad = max(cpad, nc + 1)
+        st = L.stream()
+        means = None
+        if policy & L.DIFFAUG_COLOR:
+            means = torch.empty(2 * B, dtype=F32, device=seg.device)
+            L.call("s2e_diffaug_means", L.ptr(fake), L.ptr(real), B, H, W, L.ptr(means), st)
+        out = torch.empty(2 * B, H, W, cpad, dtype=BF16, device=seg.device)
+        L.call("s2e_make_d_input_aug", L.ptr(seg), L.ptr(fake), L.ptr(real), B, nc, H, W, cpad, L.ptr(params), L.ptr(means),
+               policy, L.ptr(out), st)
+        ctx.save_for_backward(params)
+        ctx.dims = (B, nc, H, W)
+        ctx.cpad, ctx.policy = cpad, policy
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        B, nc, H, W = ctx.dims
+        dout = _c(dout)
+        dfake = None
+        if ctx.needs_input_grad[1]:
+            params, = ctx.saved_tensors
+            dfake = torch.empty(B, 1, H, W, dtype=F32, device=dout.device)
+            scratch = torch.empty(B, dtype=torch.float64, device=dout.device) if ctx.policy & L.DIFFAUG_COLOR else None
+            L.call("s2e_d_input_grad_aug", L.ptr(dout), B, nc, H, W, ctx.cpad, L.ptr(params), ctx.policy, L.ptr(scratch),
+                   L.ptr(dfake), L.stream())
+        return None, dfake, None, None, None, None
+
+
 class TanhFn(torch.autograd.Function):
     """(B,H,W,1) bf16 -> tanh -> (B,1,H,W) fp32 (generator.py:99)."""
 

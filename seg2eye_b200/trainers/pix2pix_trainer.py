@@ -31,6 +31,8 @@ class Pix2PixTrainer():
             for net in (m.netG, m.netD, m.netE, m.netG_ema, m.netE_ema):
                 if net is not None:
                     parallel.broadcast_module(net, 0)
+            if m.diffaug_state is not None:     # one seed for all ranks: rank r draws for global samples r * B + b
+                torch.distributed.broadcast(m.diffaug_state, 0)
             from .. import ops
             ops.bump_weights_epoch()
         if opt.isTrain:
@@ -42,6 +44,9 @@ class Pix2PixTrainer():
                 from .. import util
                 util.load_optimizer(self.optimizer_G, 'G', opt.which_epoch, opt, self._opt_nets('G'))
                 util.load_optimizer(self.optimizer_D, 'D', opt.which_epoch, opt, self._opt_nets('D'))
+                saved = util.load_optimizer_entry('D', opt.which_epoch, opt, 'diffaug')
+                if m.diffaug_state is not None and saved is not None:    # else: the fresh seed, counter 0
+                    m.diffaug_state.copy_(torch.tensor([saved['seed'], saved['counter']], dtype=torch.int64))
         self._graphs = False
 
     def _opt_nets(self, which):
@@ -111,6 +116,8 @@ class Pix2PixTrainer():
         m.sync_ema()
         tensors = [t for net in (m.netG, m.netD, m.netE, m.netG_ema, m.netE_ema) if net is not None
                    for t in list(net.parameters()) + list(net.buffers())]
+        if m.diffaug_state is not None:     # the warm-up steps draw: the counter is restored with the weights
+            tensors.append(m.diffaug_state)
         opts = (self.optimizer_G, self.optimizer_D)
         if multi:     # the capture set-up below runs on a side stream: no all-reduce launches from inside backward there
             self.reducer_G.remove_hooks()
@@ -264,7 +271,9 @@ class Pix2PixTrainer():
             if self.opt.isTrain:
                 from .. import util
                 util.save_optimizer(self.optimizer_G, 'G', epoch, self.opt, self._opt_nets('G'))
-                util.save_optimizer(self.optimizer_D, 'D', epoch, self.opt, self._opt_nets('D'))
+                st = self.pix2pix_model.diffaug_state
+                extra = {'diffaug': dict(seed=int(st[0]), counter=int(st[1]))} if st is not None else None
+                util.save_optimizer(self.optimizer_D, 'D', epoch, self.opt, self._opt_nets('D'), extra)
         if self.world > 1:
             torch.distributed.barrier()
 

@@ -32,11 +32,12 @@ def _named_params(nets):
     return [("%s.%s" % (tag, n), p_) for tag, net in nets if net is not None for n, p_ in net.named_parameters()]
 
 
-def save_optimizer(optimizer, label, epoch, opt, nets):
+def save_optimizer(optimizer, label, epoch, opt, nets, extra=None):
     """Beyond the reference (which restarts Adam from zero moments on --continue_train, util/util.py:195-221 saves
     networks only): `<epoch>_optim_<G|D>.pth` next to the network files -- fp32 CPU tensors keyed by parameter NAME
     ('G.up_0.conv_0.weight_orig': {'exp_avg', 'exp_avg_sq'}), plus the step count and learning rate.  Files the reference
-    never reads; its own checkpoints are untouched."""
+    never reads; its own checkpoints are untouched.  `extra`: further top-level entries of the file (the trainer stores the
+    --diff_augment generator state under 'diffaug' in the D file)."""
     save_path = os.path.join(opt.checkpoints_dir, opt.name, '%s_optim_%s.pth' % (epoch, label))
     os.makedirs(os.path.dirname(save_path), exist_ok=True)
     names = {id(p_): n for n, p_ in _named_params(nets)}
@@ -49,7 +50,16 @@ def save_optimizer(optimizer, label, epoch, opt, nets):
             s_ = optimizer.state.get(p_)
             if s_:
                 out["state"][names[id(p_)]] = {k: s_[k].detach().to('cpu') for k in ('exp_avg', 'exp_avg_sq')}
+    out.update(extra or {})
     torch.save(out, save_path)
+
+
+def load_optimizer_entry(label, epoch, opt, key):
+    """Top-level entry `key` of the file save_optimizer wrote (None when the file or the entry does not exist)."""
+    path = os.path.join(opt.checkpoints_dir, opt.name, '%s_optim_%s.pth' % (epoch, label))
+    if not os.path.exists(path):
+        return None
+    return torch.load(path, map_location='cpu').get(key)
 
 
 def load_optimizer(optimizer, label, epoch, opt, nets):
