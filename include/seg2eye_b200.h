@@ -142,6 +142,11 @@ int s2e_head_dots(const void* x_bf16, const void* wp_bf16, long long P, int Cin,
 int s2e_head_gather(const s2e_conv_t* d, const float* D, const float* bias, const float* scale, void* y_bf16, float* gan_sums,
                     void* stream);
 int s2e_head_scatter(const s2e_conv_t* d, const void* dy_bf16, void* G_bf16, void* stream);
+/* s2e_head_gather that also adds sign_sums[0] += sum sign(y) over the half b >= B/2 (the real logits of a [fake ; real]
+ * batch; y as rounded to bf16, sign(0) = 0): the statistic of --ada_target.  sign_sums: one caller-zeroed float; B even and
+ * B/2 * Ho * Wo < 2^24, so the fp32 sum of +-1 is exact whatever the order of the atomics. */
+int s2e_head_gather_signs(const s2e_conv_t* d, const float* D, const float* bias, const float* scale, void* y_bf16,
+                          float* gan_sums, float* sign_sums, void* stream);
 
 /* OIHW fp32 master weight -> bf16 tap-major.  stride 1: taps (r,s) row-major, offset (r-pad, s-pad).
  * stride 2: space-to-depth taps (a,b), a in [floor(-pad/2), floor((k-1-pad)/2)], channel (i*2+j)*Cin+ci,
@@ -351,6 +356,31 @@ int s2e_make_d_input_aug(const float* seg_nchw, const float* fake, const float* 
 int s2e_d_input_grad_aug(const void* dxin, int B, int nc, int H, int W, int Cpad, const float* params, int policy,
                          double* scratch, float* dfake, void* stream);
 
+/* Per-sample gates of the ops (--diff_augment_p, --ada_target; ADA, Karras et al., NeurIPS 2020).
+ * s2e_diffaug_draw_p writes params_out exactly as s2e_diffaug_draw does (and advances the counter by one, as it does), and
+ * opmask_out[b] = the S2E_DIFFAUG_* bits whose gate passed, op k passing iff  (double)float(r_k) < *p  with the gate words
+ *     COLOR: r6 = block 1, word 2     TRANSLATION: r7 = block 1, word 3     CUTOUT: r8 = block 2, word 0
+ * of the same Philox counter (block 2 = counter (n, ctr lo, ctr hi, 2)).  p: one double in device memory, 0 <= p <= 1; at
+ * p = 1 every gate passes, at p = 0 none does.
+ * The _masked twins of s2e_make_d_input_aug / s2e_d_input_grad_aug apply policy & opmask[b] to sample b (rows b and B + b);
+ * a sample whose colour gate is off passes its gradient through exactly.  With an empty mask they equal s2e_make_d_input /
+ * s2e_d_input_grad, with a full mask the unmasked entry points, bit for bit. */
+int s2e_diffaug_draw_p(int64_t* state, const double* p, int B, long long index_offset, int H, int W, float* params_out,
+                       int* opmask_out, void* stream);
+int s2e_make_d_input_aug_masked(const float* seg_nchw, const float* fake, const float* real, int B, int nc, int H, int W,
+                                int Cpad, const float* params, const float* means, int policy, const int* opmask, void* out,
+                                void* stream);
+int s2e_d_input_grad_aug_masked(const void* dxin, int B, int nc, int H, int W, int Cpad, const float* params, int policy,
+                                const int* opmask, double* scratch, float* dfake, void* stream);
+/* ADA's controller, one thread, device memory only (a replayed CUDA graph adapts).  step_stat: this D step's record
+ * [S_0, N_0, ..., S_{D-1}, N_{D-1}, I] (D = num_D; S_i = sum sign(real logits of scale i), N_i = their number, I = the
+ * number of real images; all-reduced over the ranks), acc: 2D + 2 doubles (the record's running sums, then the r of the last
+ * completed interval), pos: the D steps accumulated so far.  It adds step_stat into acc and, when pos + 1 reaches interval,
+ *     r = (1/D) sum_i acc[2i] / acc[2i+1],   p = min(max(p + sign(r - target) * acc[2D] / (kimg * 1000), 0), 1)   (fp64),
+ * stores r in acc[2D + 1] and resets the sums and pos to 0. */
+int s2e_ada_update(const double* step_stat, int num_D, double* acc, int* pos, double* p, double target, double kimg, int interval,
+                   void* stream);
+
 /* small fp32 linear layers: y = act(x W^T + b).  FC 16->2C (normalization.py:134-141), fc_mu/fc_var
  * (encoder.py:68-71).  in_nhwc_hw > 0: x is bf16 NHWC [M, hw, K/hw] flattened in NCHW order with LeakyReLU(0.2)
  * applied to the input first (encoder.py:64-67). */
@@ -368,6 +398,7 @@ int s2e_linear_bwd(const float* dy, const float* y, const void* x, const float* 
 #define S2E_RED_L2 4         /* (x-y)^2                                 */
 #define S2E_RED_LS 5         /* (x-target)^2          gan_mode ls       (loss.py:63-65: mse_loss against the label) */
 #define S2E_RED_BCE 6        /* BCE-with-logits(x, target)  gan_mode original (loss.py:59-62) */
+#define S2E_RED_SIGN 7       /* sign(x), sign(0) = 0 (ADA's statistic; gradient 0): exact below 2^24 elements */
 /* `target` is the constant label of the LS / BCE kinds (ignored by the others). */
 int s2e_reduce_loss(const void* x, const void* y, long long n, int x_is_f32, int kind, float coef, float target,
                     float* out, int accumulate, void* stream);

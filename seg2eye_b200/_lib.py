@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(_HERE, "_C", "libseg2eye_b200.so")
 MAX_TAPS = 16
 ACT_NONE, ACT_LRELU, ACT_RELU = 0, 1, 2
 IMPL_TC, IMPL_SIMT = 0, 1
-RED_SUM, RED_HINGE_REAL, RED_HINGE_FAKE, RED_L1, RED_L2, RED_LS, RED_BCE = 0, 1, 2, 3, 4, 5, 6
+RED_SUM, RED_HINGE_REAL, RED_HINGE_FAKE, RED_L1, RED_L2, RED_LS, RED_BCE, RED_SIGN = 0, 1, 2, 3, 4, 5, 6, 7
 DIFFAUG_COLOR, DIFFAUG_TRANSLATION, DIFFAUG_CUTOUT = 1, 2, 4
 DIFFAUG_RECORD = 6
 
@@ -55,6 +55,7 @@ _SIGS = {
     "s2e_tapconv_wgrad": [C.POINTER(ConvDesc), _P, _P, _P, _I, _P],
     "s2e_head_dots": [_P, _P, _LL, _I, _I, _P, _P],
     "s2e_head_gather": [C.POINTER(ConvDesc), _P, _P, _P, _P, _P, _P],
+    "s2e_head_gather_signs": [C.POINTER(ConvDesc), _P, _P, _P, _P, _P, _P, _P],
     "s2e_head_scatter": [C.POINTER(ConvDesc), _P, _P, _P],
     "s2e_pack_weight": [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P],
     "s2e_packed_taps": [_I, _I, _I, _I, C.POINTER(_I), C.POINTER(_I), C.POINTER(_I)],
@@ -95,6 +96,10 @@ _SIGS = {
     "s2e_diffaug_means": [_P, _P, _I, _I, _I, _P, _P],
     "s2e_make_d_input_aug": [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P],
     "s2e_d_input_grad_aug": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P],
+    "s2e_diffaug_draw_p": [_P, _P, _I, _LL, _I, _I, _P, _P, _P],
+    "s2e_make_d_input_aug_masked": [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P, _P],
+    "s2e_d_input_grad_aug_masked": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P],
+    "s2e_ada_update": [_P, _I, _P, _P, _P, _D, _D, _I, _P],
     "s2e_tanh_fwd": [_P, _LL, _P, _P],
     "s2e_tanh_bwd": [_P, _P, _LL, _P, _P],
     "s2e_linear_fwd": [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P],

@@ -671,11 +671,16 @@ __global__ void __launch_bounds__(HD_THREADS) head_dots_kernel(const bf16* __res
 //   [3h + 0] += sum y,   [3h + 1] += sum min(y - 1, 0),   [3h + 2] += sum min(-y - 1, 0)      (y as rounded to bf16)
 // i.e. the sums behind the hinge / Wasserstein terms of loss.py:58-83 (generator: -mean y_fake; discriminator: -mean min(y_real - 1, 0),
 // -mean min(-y_fake - 1, 0)), so those losses need no pass of their own over the logits.
+// SIGN (s2e_head_gather_signs): sign_sums[0] += sum sign(y) over the half b >= half_b as well (y as rounded to bf16, sign(0) = 0);
+// a block's partial sums of +-1 are integers below 2^24, so the atomics add them exactly in any order
+template <bool SIGN = false>
 __global__ void __launch_bounds__(256) head_gather_kernel(const float* __restrict__ D, const float* __restrict__ bias,
                                                           const float* __restrict__ scale, bf16* __restrict__ y, const ThinGeom g,
-                                                          long long P, float* __restrict__ gan_sums, int half_b) {
+                                                          long long P, float* __restrict__ gan_sums, int half_b,
+                                                          float* __restrict__ sign_sums = nullptr) {
   const long long p = (long long)blockIdx.x * 256 + threadIdx.x;
   float s[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  float sg = 0.f;
   if (p < P) {
     const int wo = (int)(p % g.Wo);
     const long long r = p / g.Wo;
@@ -697,6 +702,10 @@ __global__ void __launch_bounds__(256) head_gather_kernel(const float* __restric
       s[0] = h == 0 ? t0 : 0.f; s[1] = h == 0 ? t1 : 0.f; s[2] = h == 0 ? t2 : 0.f;
       s[3] = h == 3 ? t0 : 0.f; s[4] = h == 3 ? t1 : 0.f; s[5] = h == 3 ? t2 : 0.f;
     }
+    if (SIGN && b >= half_b) {
+      const float v = __bfloat162float(yb);
+      sg = (float)((v > 0.f) - (v < 0.f));
+    }
   }
   if (gan_sums) {   // kernel-uniform branch
     __shared__ float red[6][8];
@@ -711,6 +720,18 @@ __global__ void __launch_bounds__(256) head_gather_kernel(const float* __restric
 #pragma unroll
       for (int i = 0; i < 8; ++i) t += red[threadIdx.x][i];
       if (t != 0.f) atomicAdd(gan_sums + threadIdx.x, t);
+    }
+  }
+  if (SIGN) {
+    __shared__ float red_sg[8];
+    const float w = warp_sum(sg);
+    if ((threadIdx.x & 31) == 0) red_sg[threadIdx.x >> 5] = w;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      float t = 0.f;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) t += red_sg[i];
+      if (t != 0.f) atomicAdd(sign_sums, t);
     }
   }
 }
@@ -1054,6 +1075,19 @@ int s2e_head_gather(const s2e_conv_t* d, const float* D, const float* bias, cons
   if (P == 0) return S2E_OK;
   head_gather_kernel<<<(unsigned)ceil_div_ll(P, 256), 256, 0, (cudaStream_t)stream>>>(D, bias, scale, (bf16*)y, make_thin_geom(d), P, gan_sums,
                                                                                       d->B / 2);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+
+int s2e_head_gather_signs(const s2e_conv_t* d, const float* D, const float* bias, const float* scale, void* y, float* gan_sums,
+                          float* sign_sums, void* stream) {
+  S2E_REQUIRE(d && d->Cout == 1 && d->ntaps >= 1 && d->ntaps <= 16, "head_gather_signs: one output channel, <= 16 taps");
+  S2E_REQUIRE(sign_sums && d->B % 2 == 0, "head_gather_signs: the sign sum needs a [fake ; real] batch (B = %d) and a slot", d->B);
+  const long long P = (long long)d->B * d->Ho * d->Wo;
+  S2E_REQUIRE(P / 2 < (1LL << 24), "head_gather_signs: %lld real-half logits; the fp32 sign sum is exact below 2^24", P / 2);
+  if (P == 0) return S2E_OK;
+  head_gather_kernel<true><<<(unsigned)ceil_div_ll(P, 256), 256, 0, (cudaStream_t)stream>>>(D, bias, scale, (bf16*)y, make_thin_geom(d), P,
+                                                                                            gan_sums, d->B / 2, sign_sums);
   S2E_LAUNCH_CHECK();
   return S2E_OK;
 }

@@ -759,9 +759,12 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 __device__ __forceinline__ float da_unit(unsigned r) { return (float)(r >> 8) * (1.f / 16777216.f); }
 __device__ __forceinline__ int da_below(unsigned r, int n) { return (int)(((unsigned long long)r * (unsigned)n) >> 32); }
 
-// one block: thread t writes the records of samples t, t + 256, ... from the counter it read, then thread 0 advances it
+// one block: thread t writes the records of samples t, t + 256, ... from the counter it read, then thread 0 advances it.
+// GATE (s2e_diffaug_draw_p): also the per-op gates, unit(r6 | r7 | r8) < p in fp64, from block 1's spare words and block 2
+template <bool GATE>
 __global__ void __launch_bounds__(256) diffaug_draw_kernel(long long* state, int B, long long index_offset, int H, int W,
-                                                           float* __restrict__ rec) {
+                                                           float* __restrict__ rec, const double* __restrict__ prob,
+                                                           int* __restrict__ opmask) {
   const unsigned long long seed = (unsigned long long)state[0], ctr = (unsigned long long)state[1];
   const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
   const int sx = (H + 4) / 8, sy = (W + 4) / 8;    // int(H / 8 + 0.5)
@@ -777,6 +780,12 @@ __global__ void __launch_bounds__(256) diffaug_draw_kernel(long long* state, int
     o[3] = (float)(da_below(r0.w, 2 * sy + 1) - sy);
     o[4] = (float)da_below(r1.x, H + 1 - cx % 2);
     o[5] = (float)da_below(r1.y, W + 1 - cy % 2);
+    if (GATE) {
+      const uint4 r2 = philox4x32_10(make_uint4(idx, (unsigned)ctr, (unsigned)(ctr >> 32), 2u), key);
+      const double pr = *prob;
+      opmask[b] = ((double)da_unit(r1.z) < pr ? S2E_DIFFAUG_COLOR : 0) | ((double)da_unit(r1.w) < pr ? S2E_DIFFAUG_TRANSLATION : 0) |
+                  ((double)da_unit(r2.x) < pr ? S2E_DIFFAUG_CUTOUT : 0);
+    }
   }
   __syncthreads();
   if (threadIdx.x == 0) state[1] = (long long)(ctr + 1);
@@ -821,16 +830,19 @@ __device__ __forceinline__ bool da_not_cut(int i, int j, int H, int W, const flo
   return true;
 }
 
-// make_d_input_kernel with the augmentation applied while gathering: one thread per output pixel of the (2B, H, W) batch
-template <bool COLOR>
+// make_d_input_kernel with the augmentation applied while gathering: one thread per output pixel of the (2B, H, W) batch.
+// MASKED: sample b applies policy & opmask[b] (s2e_diffaug_draw_p's gates)
+template <bool COLOR, bool MASKED = false>
 __global__ void make_d_input_aug_kernel(const float* __restrict__ seg, const float* __restrict__ fake, const float* __restrict__ real,
                                         int B, int nc, int H, int W, int Cpad, long long npix, const float* __restrict__ rec,
-                                        const float* __restrict__ means, int policy, bf16* __restrict__ out) {
+                                        const float* __restrict__ means, int policy_all, bf16* __restrict__ out,
+                                        const int* __restrict__ opmask = nullptr) {
   const long long HW = (long long)H * W;
   GRID_STRIDE(p, npix) {
     const long long hw = p % HW;
     const int b2 = (int)(p / HW);
     const int b = b2 % B;
+    const int policy = MASKED ? policy_all & __ldg(opmask + b) : policy_all;
     const float* r = rec + (long long)b * S2E_DIFFAUG_RECORD;
     const int i = (int)(hw / W), j = (int)(hw % W);
     int si = i, sj = j;
@@ -844,7 +856,8 @@ __global__ void make_d_input_aug_kernel(const float* __restrict__ seg, const flo
     float img = 0.f;
     if (keep) {
       img = (b2 < B ? fake : real)[(long long)b * HW + shw];
-      if (COLOR) {   // brightness, then contrast around the brightened image's mean (saturation: identity on 1 channel)
+      if (COLOR && (!MASKED || (policy & S2E_DIFFAUG_COLOR))) {   // brightness, then contrast around the brightened image's mean
+                                                                  // (saturation: identity on 1 channel)
         const float br = __ldg(r) - 0.5f, ct = __ldg(r + 1) + 0.5f;
         const float mb = __ldg(means + b2) + br;
         img = (img + br - mb) * ct + mb;
@@ -878,10 +891,14 @@ __device__ __forceinline__ float da_grad_gather(const bf16* __restrict__ dxin, i
   if (oi < 0 || oi >= H || oj < 0 || oj >= W || !da_not_cut(oi, oj, H, W, r, policy)) return 0.f;
   return __bfloat162float(dxin[(((long long)b * H + oi) * W + oj) * Cpad + nc]);
 }
-// contrast's adjoint needs sum(g') per sample: block b reduces it in fp64
+// contrast's adjoint needs sum(g') per sample: block b reduces it in fp64 (MASKED: only where the sample's colour gate passed)
+template <bool MASKED = false>
 __global__ void __launch_bounds__(1024) d_input_grad_aug_sum_kernel(const bf16* __restrict__ dxin, int nc, int Cpad, int H, int W,
-                                                                    const float* __restrict__ rec, int policy, double* __restrict__ sums) {
+                                                                    const float* __restrict__ rec, int policy_all, double* __restrict__ sums,
+                                                                    const int* __restrict__ opmask = nullptr) {
   const int b = blockIdx.x;
+  const int policy = MASKED ? policy_all & __ldg(opmask + b) : policy_all;
+  if (MASKED && !(policy & S2E_DIFFAUG_COLOR)) return;    // block-uniform: the apply kernel passes this sample's gradient through
   const float* r = rec + (long long)b * S2E_DIFFAUG_RECORD;
   double s = 0.0;
   for (long long hw = threadIdx.x; hw < (long long)H * W; hw += blockDim.x)
@@ -889,21 +906,43 @@ __global__ void __launch_bounds__(1024) d_input_grad_aug_sum_kernel(const bf16* 
   s = block_sum_f64(s);
   if (threadIdx.x == 0) sums[b] = s;
 }
-template <bool COLOR>
+template <bool COLOR, bool MASKED = false>
 __global__ void d_input_grad_aug_kernel(const bf16* __restrict__ dxin, int B, int nc, int Cpad, int H, int W, const float* __restrict__ rec,
-                                        int policy, const double* __restrict__ sums, float* __restrict__ dfake) {
+                                        int policy_all, const double* __restrict__ sums, float* __restrict__ dfake,
+                                        const int* __restrict__ opmask = nullptr) {
   const long long HW = (long long)H * W;
   GRID_STRIDE(p, (long long)B * HW) {
     const int b = (int)(p / HW);
     const long long hw = p % HW;
+    const int policy = MASKED ? policy_all & __ldg(opmask + b) : policy_all;
     const float* r = rec + (long long)b * S2E_DIFFAUG_RECORD;
     float g = da_grad_gather(dxin, nc, Cpad, H, W, b, (int)(hw / W), (int)(hw % W), r, policy);
-    if (COLOR) {   // dfake = c g' + (1 - c) mean(g')
+    if (COLOR && (!MASKED || (policy & S2E_DIFFAUG_COLOR))) {   // dfake = c g' + (1 - c) mean(g'); a gated-off sample passes g' through
       const float ct = __ldg(r + 1) + 0.5f;
       g = fmaf(ct, g, (1.f - ct) * (float)(__ldg(sums + b) / (double)HW));
     }
     dfake[p] = g;
   }
+}
+
+// ADA's controller (Karras et al., NeurIPS 2020), one thread: the formulas are in the header next to s2e_ada_update
+__global__ void ada_update_kernel(const double* __restrict__ stat, int num_D, double* __restrict__ acc, int* __restrict__ pos,
+                                  double* __restrict__ p, double target, double kimg, int interval) {
+  const int n = 2 * num_D + 1;
+  for (int k = 0; k < n; ++k) acc[k] += stat[k];
+  const int q = *pos + 1;
+  if (q < interval) {
+    *pos = q;
+    return;
+  }
+  double r = 0.0;
+  for (int i = 0; i < num_D; ++i) r += acc[2 * i] / acc[2 * i + 1];
+  r /= (double)num_D;
+  const double sgn = (double)((r > target) - (r < target));
+  p[0] = fmin(fmax(p[0] + sgn * acc[2 * num_D] / (kimg * 1000.0), 0.0), 1.0);
+  acc[n] = r;
+  for (int k = 0; k < n; ++k) acc[k] = 0.0;
+  *pos = 0;
 }
 
 // ------------------------------------------------------------------------------------------ elementwise
@@ -1035,6 +1074,7 @@ __device__ __forceinline__ float loss_value(float a, float b, int kind, float ta
     case S2E_RED_LS: return (a - target) * (a - target);
     case S2E_RED_BCE: return fmaxf(a, 0.f) - a * target + log1pf(expf(-fabsf(a)));   // BCE with logits, stable form
     case S2E_RED_L1: return fabsf(a - b);
+    case S2E_RED_SIGN: return (float)((a > 0.f) - (a < 0.f));
     default: return (a - b) * (a - b);
   }
 }
@@ -1049,6 +1089,7 @@ __device__ __forceinline__ float loss_grad(float a, float b, int kind, float tar
       const float df = a - b;
       return df > 0.f ? 1.f : (df < 0.f ? -1.f : 0.f);
     }
+    case S2E_RED_SIGN: return 0.f;
     default: return 2.f * (a - b);
   }
 }
@@ -1541,7 +1582,16 @@ int s2e_diffaug_draw(int64_t* state, int B, long long index_offset, int H, int W
   S2E_REQUIRE(state && B >= 0 && H > 0 && W > 0 && index_offset >= 0, "diffaug_draw: bad arguments");
   S2E_REQUIRE(index_offset + B <= (1LL << 32), "diffaug_draw: sample indices must fit in 32 bits");
   S2E_REQUIRE(B == 0 || params_out, "diffaug_draw: params_out is null");
-  diffaug_draw_kernel<<<1, 256, 0, (cudaStream_t)stream>>>((long long*)state, B, index_offset, H, W, params_out);
+  diffaug_draw_kernel<false><<<1, 256, 0, (cudaStream_t)stream>>>((long long*)state, B, index_offset, H, W, params_out, nullptr, nullptr);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_diffaug_draw_p(int64_t* state, const double* p, int B, long long index_offset, int H, int W, float* params_out, int* opmask_out,
+                       void* stream) {
+  S2E_REQUIRE(state && p && B >= 0 && H > 0 && W > 0 && index_offset >= 0, "diffaug_draw_p: bad arguments");
+  S2E_REQUIRE(index_offset + B <= (1LL << 32), "diffaug_draw_p: sample indices must fit in 32 bits");
+  S2E_REQUIRE(B == 0 || (params_out && opmask_out), "diffaug_draw_p: params_out / opmask_out is null");
+  diffaug_draw_kernel<true><<<1, 256, 0, (cudaStream_t)stream>>>((long long*)state, B, index_offset, H, W, params_out, p, opmask_out);
   S2E_LAUNCH_CHECK();
   return S2E_OK;
 }
@@ -1560,7 +1610,7 @@ int s2e_make_d_input_aug(const float* seg, const float* fake, const float* real,
   const long long npix = 2LL * B * H * W;
   if (!npix) return S2E_OK;
   auto k = (policy & S2E_DIFFAUG_COLOR) ? make_d_input_aug_kernel<true> : make_d_input_aug_kernel<false>;
-  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out);
+  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out, nullptr);
   S2E_LAUNCH_CHECK();
   return S2E_OK;
 }
@@ -1578,6 +1628,44 @@ int s2e_d_input_grad_aug(const void* dxin, int B, int nc, int H, int W, int Cpad
   } else {
     d_input_grad_aug_kernel<false><<<grid1d(n), NT, 0, st>>>((const bf16*)dxin, B, nc, Cpad, H, W, params, policy, nullptr, dfake);
   }
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_make_d_input_aug_masked(const float* seg, const float* fake, const float* real, int B, int nc, int H, int W, int Cpad,
+                                const float* params, const float* means, int policy, const int* opmask, void* out, void* stream) {
+  S2E_REQUIRE(Cpad > nc, "make_d_input_aug_masked: Cpad must exceed nc");
+  S2E_REQUIRE((policy & ~S2E_DIFFAUG_ALL) == 0, "make_d_input_aug_masked: unknown policy bits %#x", policy);
+  S2E_REQUIRE(params && opmask && (means || !(policy & S2E_DIFFAUG_COLOR)), "make_d_input_aug_masked: params / opmask / means missing");
+  const long long npix = 2LL * B * H * W;
+  if (!npix) return S2E_OK;
+  auto k = (policy & S2E_DIFFAUG_COLOR) ? make_d_input_aug_kernel<true, true> : make_d_input_aug_kernel<false, true>;
+  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out, opmask);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_d_input_grad_aug_masked(const void* dxin, int B, int nc, int H, int W, int Cpad, const float* params, int policy,
+                                const int* opmask, double* scratch, float* dfake, void* stream) {
+  S2E_REQUIRE((policy & ~S2E_DIFFAUG_ALL) == 0, "d_input_grad_aug_masked: unknown policy bits %#x", policy);
+  S2E_REQUIRE(params && opmask && (scratch || !(policy & S2E_DIFFAUG_COLOR)), "d_input_grad_aug_masked: params / opmask / scratch missing");
+  const long long n = (long long)B * H * W;
+  if (!n) return S2E_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (policy & S2E_DIFFAUG_COLOR) {
+    d_input_grad_aug_sum_kernel<true><<<B, 1024, 0, st>>>((const bf16*)dxin, nc, Cpad, H, W, params, policy, scratch, opmask);
+    S2E_LAUNCH_CHECK();
+    d_input_grad_aug_kernel<true, true><<<grid1d(n), NT, 0, st>>>((const bf16*)dxin, B, nc, Cpad, H, W, params, policy, scratch, dfake,
+                                                                  opmask);
+  } else {
+    d_input_grad_aug_kernel<false, true><<<grid1d(n), NT, 0, st>>>((const bf16*)dxin, B, nc, Cpad, H, W, params, policy, nullptr, dfake,
+                                                                   opmask);
+  }
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_ada_update(const double* step_stat, int num_D, double* acc, int* pos, double* p, double target, double kimg, int interval,
+                   void* stream) {
+  S2E_REQUIRE(step_stat && acc && pos && p && num_D >= 1 && interval >= 1 && kimg > 0.0, "ada_update: bad arguments");
+  ada_update_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(step_stat, num_D, acc, pos, p, target, kimg, interval);
   S2E_LAUNCH_CHECK();
   return S2E_OK;
 }

@@ -33,6 +33,40 @@ def _diff_augment_arg(value):
         raise argparse.ArgumentTypeError(str(e))
 
 
+def _range_arg(kind, name, ok, want):
+    def check(value):
+        try:
+            v = kind(value)
+        except (TypeError, ValueError):
+            v = None
+        if v is None or not ok(v):
+            raise argparse.ArgumentTypeError('%s must be %s, got %r' % (name, want, value))
+        return v
+    return check
+
+
+_diff_augment_p_arg = _range_arg(float, '--diff_augment_p', lambda v: 0.0 <= v <= 1.0, 'in [0, 1]')
+_ada_target_arg = _range_arg(float, '--ada_target', lambda v: v == 0.0 or 0.0 < v < 1.0, '0 (off) or in (0, 1)')
+_ada_interval_arg = _range_arg(int, '--ada_interval', lambda v: v >= 1, 'a positive integer')
+_ada_kimg_arg = _range_arg(float, '--ada_kimg', lambda v: 0.0 < v < float('inf'), 'positive')
+
+
+def _ada_options(opt, policy):
+    """(p, target, interval, kimg) of --diff_augment_p / --ada_target / --ada_interval / --ada_kimg, range-checked; p
+    defaults to 1 without ADA (every op on every sample) and to 0, ADA's start value, with it."""
+    try:
+        p = _opt(opt, 'diff_augment_p', None)
+        p = None if p is None else _diff_augment_p_arg(p)
+        target = _ada_target_arg(_opt(opt, 'ada_target', 0.0))
+        interval = _ada_interval_arg(_opt(opt, 'ada_interval', 4))
+        kimg = _ada_kimg_arg(_opt(opt, 'ada_kimg', 500.0))
+    except argparse.ArgumentTypeError as e:
+        raise ValueError(str(e))
+    if not policy and (p is not None or target > 0):
+        raise ValueError('--diff_augment_p and --ada_target need --diff_augment')
+    return (1.0 if target == 0 else 0.0) if p is None else p, target, interval, kimg
+
+
 class Pix2PixModel(torch.nn.Module):
     @staticmethod
     def modify_commandline_options(parser, is_train):
@@ -44,6 +78,16 @@ class Pix2PixModel(torch.nn.Module):
                             help='beyond the reference: differentiable augmentation of everything D sees in training '
                                  '(DiffAugment), a comma-separated subset of color,translation,cutout (always applied in '
                                  'that order; empty: off)')
+        parser.add_argument('--diff_augment_p', type=_diff_augment_p_arg, default=None,
+                            help='with --diff_augment: probability with which each op is applied to each sample, 0 <= p <= 1 '
+                                 '(default: 1; with --ada_target: the start value, default 0)')
+        parser.add_argument('--ada_target', type=_ada_target_arg, default=0.0,
+                            help='with --diff_augment: adaptive augmentation (ADA): steer the probability towards '
+                                 'E[sign(D(real))] = target, 0 < target < 1 (0: off; ADA recommends 0.6)')
+        parser.add_argument('--ada_interval', type=_ada_interval_arg, default=4,
+                            help='ADA: discriminator steps between two adjustments of the probability')
+        parser.add_argument('--ada_kimg', type=_ada_kimg_arg, default=500.0,
+                            help='ADA: thousands of real images over which the probability can move from 0 to 1')
         return parser
 
     def __init__(self, opt):
@@ -51,9 +95,10 @@ class Pix2PixModel(torch.nn.Module):
         self.opt = opt
         self.ema_decay = optim.check_ema_decay(_opt(opt, 'ema_decay', 0.0))
         self.diffaug_ops, self.diffaug_policy = ops.parse_diff_augment(_opt(opt, 'diff_augment', ''))
+        self.diffaug_p, self.ada_target, self.ada_interval, self.ada_kimg = _ada_options(opt, self.diffaug_policy)
         self.netG, self.netD, self.netE = self.initialize_networks(opt)
         self.netG_ema = self.netE_ema = None
-        self.diffaug_state = None
+        self.diffaug_state = self.ada_state = None
         self._last_d_out = None
         if not opt.isTrain:
             return
@@ -62,6 +107,8 @@ class Pix2PixModel(torch.nn.Module):
             # of a captured step draw new parameters.  Held here, not by netD, whose state_dict keeps the reference's keys.
             seed = int(torch.randint(-2 ** 63, 2 ** 63 - 1, (), dtype=torch.int64))
             self.diffaug_state = torch.tensor([seed, 0], dtype=torch.int64, device=self.device())
+            if self.diffaug_p != 1.0 or self.ada_target > 0:
+                self.ada_state = self._initial_ada_state()
         if self.ema_decay > 0:
             self._initialize_ema(opt)
         if not _opt(opt, 'no_vgg_loss', True):
@@ -96,6 +143,56 @@ class Pix2PixModel(torch.nn.Module):
         for net, tag in ((self.netG, 'G'), (self.netD, 'D'), (self.netE, 'E'), (self.netG_ema, 'G_ema'), (self.netE_ema, 'E_ema')):
             if net is not None:
                 util.save_network(net, tag, epoch, self.opt)
+
+    # ------------------------------------------------------------------ augmentation probability (--diff_augment_p, --ada_target)
+    def _initial_ada_state(self):
+        """On the device, not in any state_dict: p (float64 [1]); acc, the running sums of the per-step records plus the r of
+        the last completed interval (float64 [2 num_D + 2], r = 0 before the first); pos, the D steps accumulated since
+        the last update (int32 [1]); record, this D step's [S_0, N_0, ..., S_{num_D-1}, N_{num_D-1}, I] (float64)."""
+        dev, n = self.device(), 2 * len(list(self.netD.children())) + 1
+        return {'p': torch.tensor([self.diffaug_p], dtype=torch.float64, device=dev),
+                'acc': torch.zeros(n + 1, dtype=torch.float64, device=dev),
+                'pos': torch.zeros(1, dtype=torch.int32, device=dev),
+                'record': torch.zeros(n, dtype=torch.float64, device=dev)}
+
+    def ada_checkpoint(self):
+        """The controller's state for the 'diffaug' checkpoint entry (empty without ADA: p is then the option's value)."""
+        if self.ada_target == 0:
+            return {}
+        st = self.ada_state
+        return dict(p=float(st['p']), acc=st['acc'].tolist(), pos=int(st['pos']))
+
+    def load_ada_checkpoint(self, saved):
+        """Restore what ada_checkpoint wrote; an entry without it (written before, or without ADA) leaves the start state."""
+        if self.ada_target == 0 or 'p' not in saved:
+            return
+        st = self.ada_state
+        if len(saved['acc']) != st['acc'].numel():
+            raise ValueError('checkpoint ADA state is for %d discriminator scales, this model has %d'
+                             % ((len(saved['acc']) - 2) // 2, (st['acc'].numel() - 2) // 2))
+        st['p'].fill_(saved['p'])
+        st['acc'].copy_(torch.tensor(saved['acc'], dtype=torch.float64))
+        st['pos'].fill_(saved['pos'])
+
+    def _ada_record(self, d_out, signs):
+        """This D step's record: per scale the sign sum of the real half of its logits (from the gather kernel that produced
+        them, or one S2E_RED_SIGN reduction) and their number, then the number of real images."""
+        rec = self.ada_state['record']
+        for i, scale in enumerate(d_out):
+            y = scale[-1]
+            s = signs.get(y.data_ptr())
+            if s is None:
+                flat = networks.loss._flat(y)
+                s = ops.sign_sum(flat[flat.shape[0] // 2:])
+            rec[2 * i:2 * i + 1].copy_(s)
+            rec[2 * i + 1].fill_(y.numel() // 2)
+        rec[-1].fill_(d_out[0][-1].shape[0] // 2)
+        self.add_to_loss_log('ada/p', self.ada_state['p'][0])
+        self.add_to_loss_log('ada/rt', self.ada_state['acc'][-1])
+
+    def ada_update(self):
+        """ADA's step after the D step's backward (the trainer all-reduces the record first when there are several ranks)."""
+        ops.ada_update(self.ada_state, self.ada_target, self.ada_kimg, self.ada_interval)
 
     def initialize_networks(self, opt):
         netG = networks.define_G(opt)
@@ -280,7 +377,12 @@ class Pix2PixModel(torch.nn.Module):
     def compute_discriminator_loss(self, input_semantics, real_image, target_image):
         with torch.no_grad():   # E and G run again, in training mode: BN running stats and u/v advance once more
             fake = self.generate_fake(input_semantics, real_image)[0].detach()
-        pred_fake, pred_real = self.discriminate(input_semantics, fake, target_image)
+        if self.ada_target > 0:     # --ada_target: the real logits' signs, summed in the logit heads' epilogues
+            with ops.head_sign_sums() as signs:
+                pred_fake, pred_real = self.discriminate(input_semantics, fake, target_image)
+            self._ada_record(self._last_d_out, signs)
+        else:
+            pred_fake, pred_real = self.discriminate(input_semantics, fake, target_image)
         self._last_d_out = None   # never keep an autograd graph alive across steps (CUDA-graph capture relies on it)
         return {'D/Fake': self.criterionGAN(pred_fake, False, for_discriminator=True),
                 'D/real': self.criterionGAN(pred_real, True, for_discriminator=True)}
@@ -351,13 +453,19 @@ class Pix2PixModel(torch.nn.Module):
         zero-padded to 16 so that D's first 4x4-s2 convolution is tensor-core shaped after space-to-depth.
         With --diff_augment, in training, the layout kernel's augmented twin builds it: one parameter record per sample
         pair (fake b and real b alike, so the feature-matching loss still compares aligned images), drawn for the
-        sample's global index rank * B + b."""
+        sample's global index rank * B + b.  With --diff_augment_p below 1 or --ada_target, each op of each pair is further
+        gated with the probability held on the device (ada_state['p']); otherwise today's ungated kernels run."""
         # (5 -> 16 channels for the 4-class OpenEDS maps; in general the next multiple of 16)
         cpad = -(-(input_semantics.shape[1] + 1) // 16) * 16
         if self.diffaug_policy and self.training:
             B, _, H, W = input_semantics.shape
-            params = ops.diffaug_draw(self.diffaug_state, B, parallel.rank() * B, H, W)
-            both = ops.MakeDInputAugFn.apply(input_semantics, fake_image, real_image, cpad, params, self.diffaug_policy)
+            if self.ada_state is None:
+                params = ops.diffaug_draw(self.diffaug_state, B, parallel.rank() * B, H, W)
+                both = ops.MakeDInputAugFn.apply(input_semantics, fake_image, real_image, cpad, params, self.diffaug_policy)
+            else:
+                params, opmask = ops.diffaug_draw_p(self.diffaug_state, self.ada_state['p'], B, parallel.rank() * B, H, W)
+                both = ops.MakeDInputAugMaskedFn.apply(input_semantics, fake_image, real_image, cpad, params, opmask,
+                                                       self.diffaug_policy)
         else:
             both = ops.MakeDInputFn.apply(input_semantics, fake_image, real_image, cpad)
         out = self.netD.forward_nhwc(both)

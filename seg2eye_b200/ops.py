@@ -507,11 +507,18 @@ class HeadConvFn(torch.autograd.Function):
         D = torch.empty(B * Hi * Wi, 16, dtype=F32, device=x.device)
         y = torch.empty(B, Ho, Wo, 1, dtype=BF16, device=x.device)
         # [fake ; real] batches: the sums behind GANLoss's hinge / Wasserstein terms ride in the gather kernel's epilogue
-        sums = torch.zeros(6, dtype=F32, device=x.device) if B % 2 == 0 else None
+        signs = _state.get("sign_sums")
+        signs = signs if B % 2 == 0 else None
+        sums = torch.zeros(7 if signs is not None else 6, dtype=F32, device=x.device) if B % 2 == 0 else None
         d = _desc(B, Hi, Wi, Cin, Ho, Wo, 1, taps, L.ACT_NONE)
         st = L.stream()
         L.call("s2e_head_dots", L.ptr(x), L.ptr(wp), B * Hi * Wi, Cin, len(taps), L.ptr(D), st)
-        L.call("s2e_head_gather", d, L.ptr(D), L.ptr(bias.detach() if bias is not None else None), None, L.ptr(y), L.ptr(sums), st)
+        b_ptr = L.ptr(bias.detach() if bias is not None else None)
+        if signs is None:
+            L.call("s2e_head_gather", d, L.ptr(D), b_ptr, None, L.ptr(y), L.ptr(sums), st)
+        else:     # slot 6: sum sign(y) over the real half (head_sign_sums)
+            L.call("s2e_head_gather_signs", d, L.ptr(D), b_ptr, None, L.ptr(y), L.ptr(sums), L.ptr(sums[6:]), st)
+            signs[y.data_ptr()] = sums[6:]
         ctx.cfg, ctx.has_b = cfg, bias is not None
         ctx.skip_wgrad = _state["skip_wgrad"]
         ctx.save_for_backward(x, weight)
@@ -1053,6 +1060,19 @@ def fm_pair_sums():
         _state["fm_pairs"] = prev
 
 
+@contextlib.contextmanager
+def head_sign_sums():
+    """While active, head_conv on an even ([fake ; real]) batch also sums sign(y) over the real half, in the gather kernel
+    that produces the logits (s2e_head_gather_signs).  Yields {logits data_ptr: (1,) fp32 sum} of those launches: the
+    discriminator step's statistic for --ada_target."""
+    prev = _state.get("sign_sums")
+    _state["sign_sums"] = found = {}
+    try:
+        yield found
+    finally:
+        _state["sign_sums"] = prev
+
+
 # ------------------------------------------------------------------------------------------------ elementwise / resampling
 class Upsample2xFn(torch.autograd.Function):
     @staticmethod
@@ -1334,42 +1354,101 @@ def diffaug_draw(state, B, index_offset, H, W):
     return rec
 
 
+def diffaug_draw_p(state, p, B, index_offset, H, W):
+    """diffaug_draw plus the per-op gates at probability `p` (one float64 on the device): -> the [B, 6] records, bit for
+    bit diffaug_draw's, and [B] int32 masks of the S2E_DIFFAUG_* bits whose gates passed."""
+    assert state.dtype == torch.int64 and state.numel() == 2 and state.is_contiguous()
+    assert p.dtype == torch.float64 and p.numel() == 1 and p.device == state.device
+    rec = torch.empty(B, L.DIFFAUG_RECORD, dtype=F32, device=state.device)
+    mask = torch.empty(B, dtype=torch.int32, device=state.device)
+    L.call("s2e_diffaug_draw_p", L.ptr(state), L.ptr(p), B, index_offset, H, W, L.ptr(rec), L.ptr(mask), L.stream())
+    return rec, mask
+
+
+def _d_input_aug_fwd(ctx, seg, fake, real, cpad, params, policy, opmask):
+    seg, fake, real = _c(seg.float()), _c(fake.float()), _c(real.float())
+    B, nc, H, W = seg.shape
+    assert fake.shape == (B, 1, H, W) and real.shape == (B, 1, H, W), (fake.shape, real.shape, seg.shape)
+    assert params.shape == (B, L.DIFFAUG_RECORD) and params.dtype == F32 and params.is_contiguous()
+    cpad = max(cpad, nc + 1)
+    st = L.stream()
+    means = None
+    if policy & L.DIFFAUG_COLOR:
+        means = torch.empty(2 * B, dtype=F32, device=seg.device)
+        L.call("s2e_diffaug_means", L.ptr(fake), L.ptr(real), B, H, W, L.ptr(means), st)
+    out = torch.empty(2 * B, H, W, cpad, dtype=BF16, device=seg.device)
+    if opmask is None:
+        L.call("s2e_make_d_input_aug", L.ptr(seg), L.ptr(fake), L.ptr(real), B, nc, H, W, cpad, L.ptr(params), L.ptr(means),
+               policy, L.ptr(out), st)
+        ctx.save_for_backward(params)
+    else:
+        assert opmask.shape == (B,) and opmask.dtype == torch.int32 and opmask.is_contiguous()
+        L.call("s2e_make_d_input_aug_masked", L.ptr(seg), L.ptr(fake), L.ptr(real), B, nc, H, W, cpad, L.ptr(params),
+               L.ptr(means), policy, L.ptr(opmask), L.ptr(out), st)
+        ctx.save_for_backward(params, opmask)
+    ctx.dims = (B, nc, H, W)
+    ctx.cpad, ctx.policy = cpad, policy
+    return out
+
+
+def _d_input_aug_bwd(ctx, dout):
+    B, nc, H, W = ctx.dims
+    dout = _c(dout)
+    if not ctx.needs_input_grad[1]:
+        return None
+    params, *opmask = ctx.saved_tensors
+    dfake = torch.empty(B, 1, H, W, dtype=F32, device=dout.device)
+    scratch = torch.empty(B, dtype=torch.float64, device=dout.device) if ctx.policy & L.DIFFAUG_COLOR else None
+    if not opmask:
+        L.call("s2e_d_input_grad_aug", L.ptr(dout), B, nc, H, W, ctx.cpad, L.ptr(params), ctx.policy, L.ptr(scratch),
+               L.ptr(dfake), L.stream())
+    else:
+        L.call("s2e_d_input_grad_aug_masked", L.ptr(dout), B, nc, H, W, ctx.cpad, L.ptr(params), ctx.policy, L.ptr(opmask[0]),
+               L.ptr(scratch), L.ptr(dfake), L.stream())
+    return dfake
+
+
 class MakeDInputAugFn(torch.autograd.Function):
     """MakeDInputFn with differentiable augmentation (--diff_augment): rows b and B + b use record b of `params`
     (ops.diffaug_draw); colour touches the image channel, translation and cutout every channel."""
 
     @staticmethod
     def forward(ctx, seg, fake, real, cpad, params, policy):
-        seg, fake, real = _c(seg.float()), _c(fake.float()), _c(real.float())
-        B, nc, H, W = seg.shape
-        assert fake.shape == (B, 1, H, W) and real.shape == (B, 1, H, W), (fake.shape, real.shape, seg.shape)
-        assert params.shape == (B, L.DIFFAUG_RECORD) and params.dtype == F32 and params.is_contiguous()
-        cpad = max(cpad, nc + 1)
-        st = L.stream()
-        means = None
-        if policy & L.DIFFAUG_COLOR:
-            means = torch.empty(2 * B, dtype=F32, device=seg.device)
-            L.call("s2e_diffaug_means", L.ptr(fake), L.ptr(real), B, H, W, L.ptr(means), st)
-        out = torch.empty(2 * B, H, W, cpad, dtype=BF16, device=seg.device)
-        L.call("s2e_make_d_input_aug", L.ptr(seg), L.ptr(fake), L.ptr(real), B, nc, H, W, cpad, L.ptr(params), L.ptr(means),
-               policy, L.ptr(out), st)
-        ctx.save_for_backward(params)
-        ctx.dims = (B, nc, H, W)
-        ctx.cpad, ctx.policy = cpad, policy
-        return out
+        return _d_input_aug_fwd(ctx, seg, fake, real, cpad, params, policy, None)
 
     @staticmethod
     def backward(ctx, dout):
-        B, nc, H, W = ctx.dims
-        dout = _c(dout)
-        dfake = None
-        if ctx.needs_input_grad[1]:
-            params, = ctx.saved_tensors
-            dfake = torch.empty(B, 1, H, W, dtype=F32, device=dout.device)
-            scratch = torch.empty(B, dtype=torch.float64, device=dout.device) if ctx.policy & L.DIFFAUG_COLOR else None
-            L.call("s2e_d_input_grad_aug", L.ptr(dout), B, nc, H, W, ctx.cpad, L.ptr(params), ctx.policy, L.ptr(scratch),
-                   L.ptr(dfake), L.stream())
-        return None, dfake, None, None, None, None
+        return None, _d_input_aug_bwd(ctx, dout), None, None, None, None
+
+
+class MakeDInputAugMaskedFn(torch.autograd.Function):
+    """MakeDInputAugFn with per-sample gates (--diff_augment_p, --ada_target): sample b applies policy & opmask[b]
+    (ops.diffaug_draw_p)."""
+
+    @staticmethod
+    def forward(ctx, seg, fake, real, cpad, params, opmask, policy):
+        return _d_input_aug_fwd(ctx, seg, fake, real, cpad, params, policy, opmask)
+
+    @staticmethod
+    def backward(ctx, dout):
+        return None, _d_input_aug_bwd(ctx, dout), None, None, None, None, None
+
+
+def ada_update(state, target, kimg, interval):
+    """ADA's controller step on `state` (Pix2PixModel.ada_state): adds state['record'] into state['acc'] and, every
+    `interval` calls, moves state['p'] (s2e_ada_update)."""
+    n_d = (state['record'].numel() - 1) // 2
+    L.call("s2e_ada_update", L.ptr(state['record']), n_d, L.ptr(state['acc']), L.ptr(state['pos']), L.ptr(state['p']),
+           float(target), float(kimg), int(interval), L.stream())
+
+
+def sign_sum(x):
+    """(1,) fp32 = sum sign(x) of a contiguous tensor (S2E_RED_SIGN; exact below 2^24 elements)."""
+    x = _c(x.detach())
+    assert x.numel() < 1 << 24
+    out = torch.empty(1, dtype=F32, device=x.device)
+    L.call("s2e_reduce_loss", L.ptr(x), None, x.numel(), int(x.dtype == F32), L.RED_SIGN, 1.0, 0.0, L.ptr(out), 0, L.stream())
+    return out
 
 
 class TanhFn(torch.autograd.Function):

@@ -8,7 +8,8 @@ initialised / loaded networks so that all replicas start identical, averages the
 `enable_cuda_graphs(example_batch)` captures the generator step and the discriminator step into CUDA graphs, so that a
 training iteration is a handful of graph launches instead of ~1300 kernel launches driven from Python:
   * one process: [forward + backward + Adam] is ONE graph per step;
-  * several ranks: [forward + backward] and [Adam] are two graphs with the NCCL all-reduce issued eagerly between them;
+  * several ranks: [forward + backward] and [Adam] are two graphs with the NCCL all-reduce issued eagerly between them
+    (with --ada_target also the all-reduce of the D step's sign record; the controller's update is in the [Adam] graph);
     gradients are accumulated straight into the flat all-reduce buckets (parallel.GradReducer.bind_flat_grads), the
     1/world_size factor rides on the loss."""
 import torch
@@ -33,6 +34,8 @@ class Pix2PixTrainer():
                     parallel.broadcast_module(net, 0)
             if m.diffaug_state is not None:     # one seed for all ranks: rank r draws for global samples r * B + b
                 torch.distributed.broadcast(m.diffaug_state, 0)
+            for t in (m.ada_state or {}).values():     # one augmentation probability for all ranks
+                torch.distributed.broadcast(t, 0)
             from .. import ops
             ops.bump_weights_epoch()
         if opt.isTrain:
@@ -47,6 +50,7 @@ class Pix2PixTrainer():
                 saved = util.load_optimizer_entry('D', opt.which_epoch, opt, 'diffaug')
                 if m.diffaug_state is not None and saved is not None:    # else: the fresh seed, counter 0
                     m.diffaug_state.copy_(torch.tensor([saved['seed'], saved['counter']], dtype=torch.int64))
+                    m.load_ada_checkpoint(saved)
         self._graphs = False
 
     def _opt_nets(self, which):
@@ -54,6 +58,16 @@ class Pix2PixTrainer():
         return (('G', m.netG), ('E', m.netE)) if which == 'G' else (('D', m.netD),)
 
     # ------------------------------------------------------------------ step bodies
+    def _ada_allreduce(self, which):
+        """--ada_target with several ranks: sum the D step's sign / count record over the ranks (2 num_D + 1 doubles)."""
+        m = self.pix2pix_model
+        if which == 'D' and m.ada_target > 0 and self.world > 1:
+            torch.distributed.all_reduce(m.ada_state['record'])
+
+    def _ada_update(self, which):
+        if which == 'D' and self.pix2pix_model.ada_target > 0:
+            self.pix2pix_model.ada_update()
+
     def _fb(self, which, data, scale=1.0):
         """forward + backward of one step; `scale` multiplies the loss that is differentiated (1/world_size when the
         gradients are summed across ranks afterwards), never the reported losses."""
@@ -73,6 +87,8 @@ class Pix2PixTrainer():
         opt_.zero_grad()
         losses, generated = self._fb(which, data)
         red.allreduce()
+        self._ada_allreduce(which)
+        self._ada_update(which)
         opt_.step()
         return losses, generated
 
@@ -82,6 +98,8 @@ class Pix2PixTrainer():
         red.zero_flat()
         out = self._fb(which, data, 1.0 / self.world)
         red.allreduce_flat()
+        self._ada_allreduce(which)
+        self._ada_update(which)
         opt_.step()
         return out
 
@@ -118,6 +136,7 @@ class Pix2PixTrainer():
                    for t in list(net.parameters()) + list(net.buffers())]
         if m.diffaug_state is not None:     # the warm-up steps draw: the counter is restored with the weights
             tensors.append(m.diffaug_state)
+        tensors += list((m.ada_state or {}).values())     # ... and they move the augmentation probability
         opts = (self.optimizer_G, self.optimizer_D)
         if multi:     # the capture set-up below runs on a side stream: no all-reduce launches from inside backward there
             self.reducer_G.remove_hooks()
@@ -149,6 +168,7 @@ class Pix2PixTrainer():
                 return self._split_step(which, dict(self._static))
             (self.optimizer_G if which == 'G' else self.optimizer_D).zero_grad(set_to_none=True)
             out = self._fb(which, dict(self._static))
+            self._ada_update(which)
             (self.optimizer_G if which == 'G' else self.optimizer_D).step()
             return out
 
@@ -172,13 +192,16 @@ class Pix2PixTrainer():
                     out = self._fb(which, dict(self._static), 1.0 / self.world)
                 pool = g_fb.pool()
                 red.allreduce_flat()
+                self._ada_allreduce(which)
                 g_opt = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g_opt, pool=pool):
+                    self._ada_update(which)
                     opt_.step()
             else:
                 opt_.zero_grad(set_to_none=True)
                 with torch.cuda.graph(g_fb, pool=pool):
                     out = self._fb(which, dict(self._static))
+                    self._ada_update(which)
                     opt_.step()
                 pool = g_fb.pool()
                 g_opt = None
@@ -233,6 +256,7 @@ class Pix2PixTrainer():
         g_fb.replay()
         if g_opt is not None:
             (self.reducer_G if which == 'G' else self.reducer_D).allreduce_flat()
+            self._ada_allreduce(which)
             g_opt.replay()
         if which == 'G':
             self.optimizer_G.ema_written()
@@ -272,7 +296,9 @@ class Pix2PixTrainer():
                 from .. import util
                 util.save_optimizer(self.optimizer_G, 'G', epoch, self.opt, self._opt_nets('G'))
                 st = self.pix2pix_model.diffaug_state
-                extra = {'diffaug': dict(seed=int(st[0]), counter=int(st[1]))} if st is not None else None
+                extra = None
+                if st is not None:
+                    extra = {'diffaug': dict(seed=int(st[0]), counter=int(st[1]), **self.pix2pix_model.ada_checkpoint())}
                 util.save_optimizer(self.optimizer_D, 'D', epoch, self.opt, self._opt_nets('D'), extra)
         if self.world > 1:
             torch.distributed.barrier()
