@@ -372,6 +372,58 @@ int s2e_make_d_input_aug_masked(const float* seg_nchw, const float* fake, const 
                                 void* stream);
 int s2e_d_input_grad_aug_masked(const void* dxin, int B, int nc, int H, int W, int Cpad, const float* params, int policy,
                                 const int* opmask, double* scratch, float* dfake, void* stream);
+
+/* Horizontal flip and geometric augmentation (--diff_augment xflip,geometric; ADA, Karras et al., NeurIPS 2020, the
+ * "geometric" group without rotate90 and xint).  Canonical order: color -> xflip -> geometric -> translation -> cutout.
+ *
+ * Geometry.  Pixel units, x = column, y = row, centred: xc = j - (W-1)/2, yc = i - (H-1)/2.  Sample b has one inverse
+ * 2x3 matrix M (rows b and B + b share it), mapping an output point to its source point:
+ *     M = F . S(1/s) . R(-th1) . diag(1/a, a) . R(-th2) . T(-tx W, -ty H)        (ADA's G_inv order)
+ * with R(t) = [[cos t, -sin t], [sin t, cos t]] and every factor whose gate is off the identity:
+ *     F = diag(-1, 1) (mirror),  s = 2^(0.2 n0),  a = 2^(0.2 n1),  thk = pi (2 u - 1),  (tx, ty) = 0.125 (n2, n3),
+ * composed in fp64 and rounded once to fp32 (m0 m1 m2 / m3 m4 m5 row-major, then two zero pads).
+ *
+ * Draw.  s2e_diffaug_draw_geom writes params_out and opmask bits COLOR / TRANSLATION / CUTOUT exactly as
+ * s2e_diffaug_draw_p does, geom_out [B, S2E_DIFFAUG_GEOM_RECORD] fp32, and advances the counter by one.  Words of the
+ * same Philox counter (block k = counter (n, ctr lo, ctr hi, k)); gates pass iff (double)unit(r) < q, unit as above:
+ *     block 2, words 1..3: xflip gate (q = p), mirror coin (q = 0.5), scale gate (q = p)
+ *     block 3, words 0..3: pre-rotation gate (q = p_rot), aniso gate (p), post-rotation gate (p_rot), xfrac gate (p)
+ *     block 4: Box-Muller of words 0, 1 -> (n0, n1); th1 from word 2, th2 from word 3
+ *     block 5: Box-Muller of words 0, 1 -> (n2, n3)
+ * p_rot = 1 - sqrt(max(1 - p, 0)) (fp64).  Box-Muller in fp64: u = ((r0 >> 8) + 0.5) 2^-24, v likewise from r1,
+ * n0 = sqrt(-2 ln u) cos(2 pi v), n1 = sqrt(-2 ln u) sin(2 pi v); |n| <= 5.9, so s and a lie in about [0.44, 2.3].
+ * Every parameter is drawn whatever the gates.  opmask bit XFLIP: the mirror is applied (xflip gate and coin);
+ * bit GEOMETRIC: some of the five geometric gates passed.
+ *
+ * Sampling (s2e_make_d_input_aug_geom; sample b applies policy & opmask[b], and M without F when the policy lacks XFLIP).
+ * A sample with neither new bit takes s2e_make_d_input_aug_masked's path, bit for bit; XFLIP alone reads column
+ * W-1-j exactly.  Otherwise an output pixel is first moved by cutout and translation to the warped-image position
+ * (si, sj) as above (zero outside), then, in fp32 without contraction,
+ *     X = ((m0 xc + m1 yc) + m2) + (W-1)/2,   Y = ((m3 xc + m4 yc) + m5) + (H-1)/2,   xc = sj - (W-1)/2, yc = si - (H-1)/2;
+ * the image channel is sampled bilinearly at the taps floor(X) + {0, 1}, floor(Y) + {0, 1} (weights from the fp32
+ * fractions), the label channels at the nearest tap floor(X + 0.5), floor(Y + 0.5) (labels stay one-hot); every tap
+ * index k is folded into [0, n) by reflection, fold(k, n): m = 2(n-1), k' = k mod m, k' < n ? k' : m - k' (torch's
+ * 'reflect', repeated).  Colour is applied to the sampled value, then one rounding to bf16.  Needs H, W >= 2.
+ * Departures from ADA, deliberate: labels are sampled nearest, not warped alike, and there is no 2x oversampling with
+ * wavelet filters.
+ *
+ * Adjoint (s2e_d_input_grad_aug_geom, the fake image): with h the gathered gradient of s2e_d_input_grad_aug at the
+ * warped-image position, dfake = Warp^T(h) (mirror alone: h at column W-1-j), then colour's c dfake + (1 - c) sum(h)/HW.
+ * Warp^T is a gather with a fixed summation order (deterministic, no atomics): each source pixel enumerates its mirror
+ * images +-s + 2k(n-1) within the bounding box of M (output rect) widened by two pixels (the second tap, and margin for
+ * the fp32 coordinates), scans the integer box of
+ * M^-1 (image + [-1, 1]^2) widened by one pixel (fp64), and accepts a candidate only if the forward's fp32 taps land on it. */
+#define S2E_DIFFAUG_XFLIP 8
+#define S2E_DIFFAUG_GEOMETRIC 16
+#define S2E_DIFFAUG_ALL_GEOM 31
+#define S2E_DIFFAUG_GEOM_RECORD 8
+int s2e_diffaug_draw_geom(int64_t* state, const double* p, int B, long long index_offset, int H, int W, float* params_out,
+                          float* geom_out, int* opmask_out, void* stream);
+int s2e_make_d_input_aug_geom(const float* seg_nchw, const float* fake, const float* real, int B, int nc, int H, int W,
+                              int Cpad, const float* params, const float* means, int policy, const int* opmask,
+                              const float* geom, void* out, void* stream);
+int s2e_d_input_grad_aug_geom(const void* dxin, int B, int nc, int H, int W, int Cpad, const float* params, int policy,
+                              const int* opmask, const float* geom, double* scratch, float* dfake, void* stream);
 /* ADA's controller, one thread, device memory only (a replayed CUDA graph adapts).  step_stat: this D step's record
  * [S_0, N_0, ..., S_{D-1}, N_{D-1}, I] (D = num_D; S_i = sum sign(real logits of scale i), N_i = their number, I = the
  * number of real images; all-reduced over the ranks), acc: 2D + 2 doubles (the record's running sums, then the r of the last

@@ -14,7 +14,8 @@ ACT_NONE, ACT_LRELU, ACT_RELU = 0, 1, 2
 IMPL_TC, IMPL_SIMT = 0, 1
 RED_SUM, RED_HINGE_REAL, RED_HINGE_FAKE, RED_L1, RED_L2, RED_LS, RED_BCE, RED_SIGN = 0, 1, 2, 3, 4, 5, 6, 7
 DIFFAUG_COLOR, DIFFAUG_TRANSLATION, DIFFAUG_CUTOUT = 1, 2, 4
-DIFFAUG_RECORD = 6
+DIFFAUG_XFLIP, DIFFAUG_GEOMETRIC = 8, 16
+DIFFAUG_RECORD, DIFFAUG_GEOM_RECORD = 6, 8
 
 
 class ConvDesc(C.Structure):
@@ -99,6 +100,9 @@ _SIGS = {
     "s2e_diffaug_draw_p": [_P, _P, _I, _LL, _I, _I, _P, _P, _P],
     "s2e_make_d_input_aug_masked": [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P, _P],
     "s2e_d_input_grad_aug_masked": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P],
+    "s2e_diffaug_draw_geom": [_P, _P, _I, _LL, _I, _I, _P, _P, _P, _P],
+    "s2e_make_d_input_aug_geom": [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P, _P, _P, _P],
+    "s2e_d_input_grad_aug_geom": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _P],
     "s2e_ada_update": [_P, _I, _P, _P, _P, _D, _D, _I, _P],
     "s2e_tanh_fwd": [_P, _LL, _P, _P],
     "s2e_tanh_bwd": [_P, _P, _LL, _P, _P],

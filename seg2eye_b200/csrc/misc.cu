@@ -759,12 +759,56 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 __device__ __forceinline__ float da_unit(unsigned r) { return (float)(r >> 8) * (1.f / 16777216.f); }
 __device__ __forceinline__ int da_below(unsigned r, int n) { return (int)(((unsigned long long)r * (unsigned)n) >> 32); }
 
+// Box-Muller in fp64 on two words, u = ((r >> 8) + 0.5) 2^-24 > 0 so that log(u) is finite
+__device__ __forceinline__ double2 da_normal2(unsigned ru, unsigned rv) {
+  const double u = ((double)(ru >> 8) + 0.5) * (1.0 / 16777216.0), v = ((double)(rv >> 8) + 0.5) * (1.0 / 16777216.0);
+  const double r = sqrt(-2.0 * log(u));
+  double sn, cs;
+  sincospi(2.0 * v, &sn, &cs);
+  return make_double2(r * cs, r * sn);
+}
+
+// the geometric record of one sample (s2e_diffaug_draw_geom's formulas in the header): M in fp64, rounded once to fp32
+__device__ void da_draw_geom(uint4 c, uint2 key, uint4 r2, double p, int H, int W, float* __restrict__ m, int& bits) {
+  c.w = 3u;
+  const uint4 r3 = philox4x32_10(c, key);
+  c.w = 4u;
+  const uint4 r4 = philox4x32_10(c, key);
+  c.w = 5u;
+  const uint4 r5 = philox4x32_10(c, key);
+  const double p_rot = 1.0 - sqrt(fmax(1.0 - p, 0.0));
+  const bool mirror = (double)da_unit(r2.y) < p && (double)da_unit(r2.z) < 0.5;
+  const bool g_s = (double)da_unit(r2.w) < p, g_r1 = (double)da_unit(r3.x) < p_rot, g_a = (double)da_unit(r3.y) < p;
+  const bool g_r2 = (double)da_unit(r3.z) < p_rot, g_t = (double)da_unit(r3.w) < p;
+  const double2 n01 = da_normal2(r4.x, r4.y), n23 = da_normal2(r5.x, r5.y);
+  const double is = g_s ? exp2(-0.2 * n01.x) : 1.0, ia = g_a ? exp2(-0.2 * n01.y) : 1.0;
+  const double t1 = g_r1 ? 2.0 * (double)da_unit(r4.z) - 1.0 : 0.0, t2 = g_r2 ? 2.0 * (double)da_unit(r4.w) - 1.0 : 0.0;
+  double s1, c1, s2, c2;
+  sincospi(t1, &s1, &c1);
+  sincospi(t2, &s2, &c2);
+  // A = F S(1/s) R(-th1) diag(1/a, a) R(-th2), R(-t) = [[cos t, sin t], [-sin t, cos t]]
+  const double b00 = c1 * ia, b01 = s1 / ia, b10 = -s1 * ia, b11 = c1 / ia;          // R(-th1) diag(1/a, a)
+  const double f = mirror ? -is : is;
+  const double a00 = f * (b00 * c2 - b01 * s2), a01 = f * (b00 * s2 + b01 * c2);
+  const double a10 = is * (b10 * c2 - b11 * s2), a11 = is * (b10 * s2 + b11 * c2);
+  const double dx = g_t ? -0.125 * n23.x * (double)W : 0.0, dy = g_t ? -0.125 * n23.y * (double)H : 0.0;
+  m[0] = (float)a00;
+  m[1] = (float)a01;
+  m[2] = (float)(a00 * dx + a01 * dy);
+  m[3] = (float)a10;
+  m[4] = (float)a11;
+  m[5] = (float)(a10 * dx + a11 * dy);
+  m[6] = m[7] = 0.f;
+  bits = (mirror ? S2E_DIFFAUG_XFLIP : 0) | ((g_s || g_r1 || g_a || g_r2 || g_t) ? S2E_DIFFAUG_GEOMETRIC : 0);
+}
+
 // one block: thread t writes the records of samples t, t + 256, ... from the counter it read, then thread 0 advances it.
 // GATE (s2e_diffaug_draw_p): also the per-op gates, unit(r6 | r7 | r8) < p in fp64, from block 1's spare words and block 2
-template <bool GATE>
+// GEOM (s2e_diffaug_draw_geom, with GATE): also the mirror and geometric records and bits, from blocks 2 to 5
+template <bool GATE, bool GEOM = false>
 __global__ void __launch_bounds__(256) diffaug_draw_kernel(long long* state, int B, long long index_offset, int H, int W,
                                                            float* __restrict__ rec, const double* __restrict__ prob,
-                                                           int* __restrict__ opmask) {
+                                                           int* __restrict__ opmask, float* __restrict__ geom = nullptr) {
   const unsigned long long seed = (unsigned long long)state[0], ctr = (unsigned long long)state[1];
   const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
   const int sx = (H + 4) / 8, sy = (W + 4) / 8;    // int(H / 8 + 0.5)
@@ -783,8 +827,15 @@ __global__ void __launch_bounds__(256) diffaug_draw_kernel(long long* state, int
     if (GATE) {
       const uint4 r2 = philox4x32_10(make_uint4(idx, (unsigned)ctr, (unsigned)(ctr >> 32), 2u), key);
       const double pr = *prob;
-      opmask[b] = ((double)da_unit(r1.z) < pr ? S2E_DIFFAUG_COLOR : 0) | ((double)da_unit(r1.w) < pr ? S2E_DIFFAUG_TRANSLATION : 0) |
-                  ((double)da_unit(r2.x) < pr ? S2E_DIFFAUG_CUTOUT : 0);
+      int bits = ((double)da_unit(r1.z) < pr ? S2E_DIFFAUG_COLOR : 0) | ((double)da_unit(r1.w) < pr ? S2E_DIFFAUG_TRANSLATION : 0) |
+                 ((double)da_unit(r2.x) < pr ? S2E_DIFFAUG_CUTOUT : 0);
+      if constexpr (GEOM) {
+        int gbits;
+        da_draw_geom(make_uint4(idx, (unsigned)ctr, (unsigned)(ctr >> 32), 0u), key, r2, pr, H, W,
+                     geom + (long long)b * S2E_DIFFAUG_GEOM_RECORD, gbits);
+        bits |= gbits;
+      }
+      opmask[b] = bits;
     }
   }
   __syncthreads();
@@ -830,13 +881,41 @@ __device__ __forceinline__ bool da_not_cut(int i, int j, int H, int W, const flo
   return true;
 }
 
+// reflection of a tap index into [0, n), n >= 2: torch's 'reflect' padding, repeated
+__device__ __forceinline__ int da_fold(int k, int n) {
+  const int m = 2 * (n - 1);
+  int q = k % m;
+  if (q < 0) q += m;
+  return q < n ? q : m - q;
+}
+// the source point of warped-image position (si, sj) in pixel coordinates, fp32 without contraction (the header's X, Y)
+__device__ __forceinline__ void da_warp(const float* m, int si, int sj, int H, int W, float& X, float& Y) {
+  const float hx = 0.5f * (float)(W - 1), hy = 0.5f * (float)(H - 1);
+  const float xc = __fsub_rn((float)sj, hx), yc = __fsub_rn((float)si, hy);
+  X = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], xc), __fmul_rn(m[1], yc)), m[2]), hx);
+  Y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[3], xc), __fmul_rn(m[4], yc)), m[5]), hy);
+}
+// sample b's M for its policy: s2e_diffaug_draw_geom folds the mirror into row 0 whenever the coin applied it, so a policy
+// without XFLIP negates that row back (exact)
+__device__ __forceinline__ void da_load_m(const float* __restrict__ geom, int b, int policy, int mask, float* m) {
+  const float* g = geom + (long long)b * S2E_DIFFAUG_GEOM_RECORD;
+  const float f = ((mask & S2E_DIFFAUG_XFLIP) && !(policy & S2E_DIFFAUG_XFLIP)) ? -1.f : 1.f;
+  m[0] = f * __ldg(g);
+  m[1] = f * __ldg(g + 1);
+  m[2] = f * __ldg(g + 2);
+  m[3] = __ldg(g + 3);
+  m[4] = __ldg(g + 4);
+  m[5] = __ldg(g + 5);
+}
+
 // make_d_input_kernel with the augmentation applied while gathering: one thread per output pixel of the (2B, H, W) batch.
 // MASKED: sample b applies policy & opmask[b] (s2e_diffaug_draw_p's gates)
-template <bool COLOR, bool MASKED = false>
+// GEOM (with MASKED): also XFLIP / GEOMETRIC with geom's matrices (s2e_diffaug_draw_geom)
+template <bool COLOR, bool MASKED = false, bool GEOM = false>
 __global__ void make_d_input_aug_kernel(const float* __restrict__ seg, const float* __restrict__ fake, const float* __restrict__ real,
                                         int B, int nc, int H, int W, int Cpad, long long npix, const float* __restrict__ rec,
                                         const float* __restrict__ means, int policy_all, bf16* __restrict__ out,
-                                        const int* __restrict__ opmask = nullptr) {
+                                        const int* __restrict__ opmask = nullptr, const float* __restrict__ geom = nullptr) {
   const long long HW = (long long)H * W;
   GRID_STRIDE(p, npix) {
     const long long hw = p % HW;
@@ -851,11 +930,28 @@ __global__ void make_d_input_aug_kernel(const float* __restrict__ seg, const flo
       sj += (int)__ldg(r + 3);
     }
     const bool keep = si >= 0 && si < H && sj >= 0 && sj < W && da_not_cut(i, j, H, W, r, policy);
-    const long long shw = keep ? (long long)si * W + sj : 0;
-    const float* sp = seg + (long long)b * nc * HW + shw;
+    long long shw = keep ? (long long)si * W + sj : 0;
     float img = 0.f;
+    bool warped = false;
+    if constexpr (GEOM) {
+      if (keep && (policy & S2E_DIFFAUG_GEOMETRIC)) {   // labels at the nearest tap, the image bilinear, taps reflected
+        float m[6], X, Y;
+        da_load_m(geom, b, policy, __ldg(opmask + b), m);
+        da_warp(m, si, sj, H, W, X, Y);
+        shw = (long long)da_fold((int)floorf(Y + 0.5f), H) * W + da_fold((int)floorf(X + 0.5f), W);
+        const float x0 = floorf(X), y0 = floorf(Y), fx = X - x0, fy = Y - y0;
+        const int c0 = da_fold((int)x0, W), c1 = da_fold((int)x0 + 1, W);
+        const float* row0 = (b2 < B ? fake : real) + (long long)b * HW + (long long)da_fold((int)y0, H) * W;
+        const float* row1 = (b2 < B ? fake : real) + (long long)b * HW + (long long)da_fold((int)y0 + 1, H) * W;
+        img = (1.f - fy) * ((1.f - fx) * row0[c0] + fx * row0[c1]) + fy * ((1.f - fx) * row1[c0] + fx * row1[c1]);
+        warped = true;
+      } else if (keep && (policy & S2E_DIFFAUG_XFLIP)) {
+        shw = (long long)si * W + (W - 1 - sj);
+      }
+    }
+    const float* sp = seg + (long long)b * nc * HW + shw;
     if (keep) {
-      img = (b2 < B ? fake : real)[(long long)b * HW + shw];
+      if (!warped) img = (b2 < B ? fake : real)[(long long)b * HW + shw];
       if (COLOR && (!MASKED || (policy & S2E_DIFFAUG_COLOR))) {   // brightness, then contrast around the brightened image's mean
                                                                   // (saturation: identity on 1 channel)
         const float br = __ldg(r) - 0.5f, ct = __ldg(r + 1) + 0.5f;
@@ -906,17 +1002,74 @@ __global__ void __launch_bounds__(1024) d_input_grad_aug_sum_kernel(const bf16* 
   s = block_sum_f64(s);
   if (threadIdx.x == 0) sums[b] = s;
 }
-template <bool COLOR, bool MASKED = false>
+// the unfolded images k = s0 + 2 t (n-1), s0 in {s, -s} (once when s is 0 or n-1), that lie in [lo, hi]: callback f(k)
+template <class Fn>
+__device__ __forceinline__ void da_for_images(int s, int n, double lo, double hi, Fn&& f) {
+  const int period = 2 * (n - 1);
+  for (int fam = 0; fam < ((s == 0 || s == n - 1) ? 1 : 2); ++fam) {
+    const int s0 = fam ? -s : s;
+    const int t0 = (int)ceil((lo - s0) / period), t1 = (int)floor((hi - s0) / period);
+    for (int t = t0; t <= t1; ++t) f(s0 + t * period);
+  }
+}
+// Warp^T(h) at source pixel (sr, sc) of sample b: every (warped-image position, bilinear tap) pair whose folded tap is
+// (sr, sc), summed in a fixed order.  The boxes only bound the search; the forward's own fp32 taps decide.
+__device__ float da_warp_adjoint(const bf16* __restrict__ dxin, int nc, int Cpad, int H, int W, int b, int sr, int sc,
+                                 const float* r, int policy, const float* m) {
+  const double hx = 0.5 * (W - 1), hy = 0.5 * (H - 1);
+  const double m0 = m[0], m1 = m[1], m2 = m[2], m3 = m[3], m4 = m[4], m5 = m[5];
+  // reach: the taps of M (output rect), widened
+  const double ex = fabs(m0) * hx + fabs(m1) * hy, ey = fabs(m3) * hx + fabs(m4) * hy;
+  const double xlo = m2 + hx - ex - 2.0, xhi = m2 + hx + ex + 2.0, ylo = m5 + hy - ey - 2.0, yhi = m5 + hy + ey + 2.0;
+  const double det = m0 * m4 - m1 * m3;
+  const double i00 = m4 / det, i01 = -m1 / det, i10 = -m3 / det, i11 = m0 / det;
+  const double bx = fabs(i00) + fabs(i01) + 1.0, by = fabs(i10) + fabs(i11) + 1.0;    // M^-1 ([-1, 1]^2), + 1 pixel
+  float acc = 0.f;
+  da_for_images(sr, H, ylo, yhi, [&](int R) {
+    da_for_images(sc, W, xlo, xhi, [&](int C) {
+      const double px = C - hx - m2, py = R - hy - m5;
+      const double qx = i00 * px + i01 * py + hx, qy = i10 * px + i11 * py + hy;
+      const int j0 = max(0, (int)ceil(qx - bx)), j1 = min(W - 1, (int)floor(qx + bx));
+      const int q0 = max(0, (int)ceil(qy - by)), q1 = min(H - 1, (int)floor(qy + by));
+      for (int qi = q0; qi <= q1; ++qi)
+        for (int qj = j0; qj <= j1; ++qj) {
+          float X, Y;
+          da_warp(m, qi, qj, H, W, X, Y);
+          const float x0 = floorf(X), y0 = floorf(Y);
+          const int dx = C - (int)x0, dy = R - (int)y0;
+          if ((unsigned)dx > 1u || (unsigned)dy > 1u) continue;
+          const float fx = X - x0, fy = Y - y0;
+          const float w = (dy ? fy : 1.f - fy) * (dx ? fx : 1.f - fx);
+          acc = fmaf(w, da_grad_gather(dxin, nc, Cpad, H, W, b, qi, qj, r, policy), acc);
+        }
+    });
+  });
+  return acc;
+}
+
+template <bool COLOR, bool MASKED = false, bool GEOM = false>
 __global__ void d_input_grad_aug_kernel(const bf16* __restrict__ dxin, int B, int nc, int Cpad, int H, int W, const float* __restrict__ rec,
                                         int policy_all, const double* __restrict__ sums, float* __restrict__ dfake,
-                                        const int* __restrict__ opmask = nullptr) {
+                                        const int* __restrict__ opmask = nullptr, const float* __restrict__ geom = nullptr) {
   const long long HW = (long long)H * W;
   GRID_STRIDE(p, (long long)B * HW) {
     const int b = (int)(p / HW);
     const long long hw = p % HW;
     const int policy = MASKED ? policy_all & __ldg(opmask + b) : policy_all;
     const float* r = rec + (long long)b * S2E_DIFFAUG_RECORD;
-    float g = da_grad_gather(dxin, nc, Cpad, H, W, b, (int)(hw / W), (int)(hw % W), r, policy);
+    float g;
+    if constexpr (GEOM) {
+      const int i = (int)(hw / W), j = (int)(hw % W);
+      if (policy & S2E_DIFFAUG_GEOMETRIC) {
+        float m[6];
+        da_load_m(geom, b, policy, __ldg(opmask + b), m);
+        g = da_warp_adjoint(dxin, nc, Cpad, H, W, b, i, j, r, policy, m);
+      } else {
+        g = da_grad_gather(dxin, nc, Cpad, H, W, b, i, (policy & S2E_DIFFAUG_XFLIP) ? W - 1 - j : j, r, policy);
+      }
+    } else {
+      g = da_grad_gather(dxin, nc, Cpad, H, W, b, (int)(hw / W), (int)(hw % W), r, policy);
+    }
     if (COLOR && (!MASKED || (policy & S2E_DIFFAUG_COLOR))) {   // dfake = c g' + (1 - c) mean(g'); a gated-off sample passes g' through
       const float ct = __ldg(r + 1) + 0.5f;
       g = fmaf(ct, g, (1.f - ct) * (float)(__ldg(sums + b) / (double)HW));
@@ -1610,7 +1763,8 @@ int s2e_make_d_input_aug(const float* seg, const float* fake, const float* real,
   const long long npix = 2LL * B * H * W;
   if (!npix) return S2E_OK;
   auto k = (policy & S2E_DIFFAUG_COLOR) ? make_d_input_aug_kernel<true> : make_d_input_aug_kernel<false>;
-  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out, nullptr);
+  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out, nullptr,
+                                                   nullptr);
   S2E_LAUNCH_CHECK();
   return S2E_OK;
 }
@@ -1639,7 +1793,8 @@ int s2e_make_d_input_aug_masked(const float* seg, const float* fake, const float
   const long long npix = 2LL * B * H * W;
   if (!npix) return S2E_OK;
   auto k = (policy & S2E_DIFFAUG_COLOR) ? make_d_input_aug_kernel<true, true> : make_d_input_aug_kernel<false, true>;
-  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out, opmask);
+  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out, opmask,
+                                                   nullptr);
   S2E_LAUNCH_CHECK();
   return S2E_OK;
 }
@@ -1658,6 +1813,53 @@ int s2e_d_input_grad_aug_masked(const void* dxin, int B, int nc, int H, int W, i
   } else {
     d_input_grad_aug_kernel<false, true><<<grid1d(n), NT, 0, st>>>((const bf16*)dxin, B, nc, Cpad, H, W, params, policy, nullptr, dfake,
                                                                    opmask);
+  }
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_diffaug_draw_geom(int64_t* state, const double* p, int B, long long index_offset, int H, int W, float* params_out,
+                          float* geom_out, int* opmask_out, void* stream) {
+  S2E_REQUIRE(state && p && B >= 0 && H > 0 && W > 0 && index_offset >= 0, "diffaug_draw_geom: bad arguments");
+  S2E_REQUIRE(index_offset + B <= (1LL << 32), "diffaug_draw_geom: sample indices must fit in 32 bits");
+  S2E_REQUIRE(B == 0 || (params_out && geom_out && opmask_out), "diffaug_draw_geom: params_out / geom_out / opmask_out is null");
+  diffaug_draw_kernel<true, true><<<1, 256, 0, (cudaStream_t)stream>>>((long long*)state, B, index_offset, H, W, params_out, p,
+                                                                        opmask_out, geom_out);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_make_d_input_aug_geom(const float* seg, const float* fake, const float* real, int B, int nc, int H, int W, int Cpad,
+                              const float* params, const float* means, int policy, const int* opmask, const float* geom, void* out,
+                              void* stream) {
+  S2E_REQUIRE(Cpad > nc, "make_d_input_aug_geom: Cpad must exceed nc");
+  S2E_REQUIRE((policy & ~S2E_DIFFAUG_ALL_GEOM) == 0, "make_d_input_aug_geom: unknown policy bits %#x", policy);
+  S2E_REQUIRE(!(policy & S2E_DIFFAUG_GEOMETRIC) || (H >= 2 && W >= 2), "make_d_input_aug_geom: geometric needs H, W >= 2");
+  S2E_REQUIRE(params && opmask && geom && (means || !(policy & S2E_DIFFAUG_COLOR)),
+              "make_d_input_aug_geom: params / opmask / geom / means missing");
+  const long long npix = 2LL * B * H * W;
+  if (!npix) return S2E_OK;
+  auto k = (policy & S2E_DIFFAUG_COLOR) ? make_d_input_aug_kernel<true, true, true> : make_d_input_aug_kernel<false, true, true>;
+  k<<<grid1d(npix), NT, 0, (cudaStream_t)stream>>>(seg, fake, real, B, nc, H, W, Cpad, npix, params, means, policy, (bf16*)out, opmask,
+                                                   geom);
+  S2E_LAUNCH_CHECK();
+  return S2E_OK;
+}
+int s2e_d_input_grad_aug_geom(const void* dxin, int B, int nc, int H, int W, int Cpad, const float* params, int policy,
+                              const int* opmask, const float* geom, double* scratch, float* dfake, void* stream) {
+  S2E_REQUIRE((policy & ~S2E_DIFFAUG_ALL_GEOM) == 0, "d_input_grad_aug_geom: unknown policy bits %#x", policy);
+  S2E_REQUIRE(!(policy & S2E_DIFFAUG_GEOMETRIC) || (H >= 2 && W >= 2), "d_input_grad_aug_geom: geometric needs H, W >= 2");
+  S2E_REQUIRE(params && opmask && geom && (scratch || !(policy & S2E_DIFFAUG_COLOR)),
+              "d_input_grad_aug_geom: params / opmask / geom / scratch missing");
+  const long long n = (long long)B * H * W;
+  if (!n) return S2E_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (policy & S2E_DIFFAUG_COLOR) {
+    d_input_grad_aug_sum_kernel<true><<<B, 1024, 0, st>>>((const bf16*)dxin, nc, Cpad, H, W, params, policy, scratch, opmask);
+    S2E_LAUNCH_CHECK();
+    d_input_grad_aug_kernel<true, true, true><<<grid1d(n), NT, 0, st>>>((const bf16*)dxin, B, nc, Cpad, H, W, params, policy, scratch,
+                                                                        dfake, opmask, geom);
+  } else {
+    d_input_grad_aug_kernel<false, true, true><<<grid1d(n), NT, 0, st>>>((const bf16*)dxin, B, nc, Cpad, H, W, params, policy, nullptr,
+                                                                         dfake, opmask, geom);
   }
   S2E_LAUNCH_CHECK();
   return S2E_OK;

@@ -76,8 +76,9 @@ class Pix2PixModel(torch.nn.Module):
                                  'this decay, 0 <= decay < 1 (0: off); inference uses it, saved as <epoch>_net_G_ema.pth')
         parser.add_argument('--diff_augment', type=_diff_augment_arg, default='',
                             help='beyond the reference: differentiable augmentation of everything D sees in training '
-                                 '(DiffAugment), a comma-separated subset of color,translation,cutout (always applied in '
-                                 'that order; empty: off)')
+                                 '(DiffAugment, ADA), a comma-separated subset of color,xflip,geometric,translation,cutout '
+                                 '(always applied in that order; xflip: horizontal mirror, geometric: ADA\'s scaling, '
+                                 'rotations and fractional translation as one bilinear warp with reflect padding; empty: off)')
         parser.add_argument('--diff_augment_p', type=_diff_augment_p_arg, default=None,
                             help='with --diff_augment: probability with which each op is applied to each sample, 0 <= p <= 1 '
                                  '(default: 1; with --ada_target: the start value, default 0)')
@@ -107,7 +108,9 @@ class Pix2PixModel(torch.nn.Module):
             # of a captured step draw new parameters.  Held here, not by netD, whose state_dict keeps the reference's keys.
             seed = int(torch.randint(-2 ** 63, 2 ** 63 - 1, (), dtype=torch.int64))
             self.diffaug_state = torch.tensor([seed, 0], dtype=torch.int64, device=self.device())
-            if self.diffaug_p != 1.0 or self.ada_target > 0:
+            # p on the device: gated ops (--diff_augment_p below 1, ADA), and the mirror / geometric ops, whose draw is
+            # always gated (p = 1 without ADA: every gate passes and the mirror is a fair coin)
+            if self.diffaug_p != 1.0 or self.ada_target > 0 or self.diffaug_policy & ops.DIFFAUG_GEOM_OPS:
                 self.ada_state = self._initial_ada_state()
         if self.ema_decay > 0:
             self._initialize_ema(opt)
@@ -454,12 +457,18 @@ class Pix2PixModel(torch.nn.Module):
         With --diff_augment, in training, the layout kernel's augmented twin builds it: one parameter record per sample
         pair (fake b and real b alike, so the feature-matching loss still compares aligned images), drawn for the
         sample's global index rank * B + b.  With --diff_augment_p below 1 or --ada_target, each op of each pair is further
-        gated with the probability held on the device (ada_state['p']); otherwise today's ungated kernels run."""
+        gated with the probability held on the device (ada_state['p']); otherwise today's ungated kernels run.  A policy
+        with xflip or geometric always takes the gated path with the mirror and the per-sample warp matrices."""
         # (5 -> 16 channels for the 4-class OpenEDS maps; in general the next multiple of 16)
         cpad = -(-(input_semantics.shape[1] + 1) // 16) * 16
         if self.diffaug_policy and self.training:
             B, _, H, W = input_semantics.shape
-            if self.ada_state is None:
+            if self.diffaug_policy & ops.DIFFAUG_GEOM_OPS:
+                params, geom, opmask = ops.diffaug_draw_geom(self.diffaug_state, self.ada_state['p'], B, parallel.rank() * B,
+                                                             H, W)
+                both = ops.MakeDInputAugGeomFn.apply(input_semantics, fake_image, real_image, cpad, params, opmask, geom,
+                                                     self.diffaug_policy)
+            elif self.ada_state is None:
                 params = ops.diffaug_draw(self.diffaug_state, B, parallel.rank() * B, H, W)
                 both = ops.MakeDInputAugFn.apply(input_semantics, fake_image, real_image, cpad, params, self.diffaug_policy)
             else:

@@ -1330,12 +1330,14 @@ class MakeDInputFn(torch.autograd.Function):
         return None, dfake, None, None
 
 
-DIFFAUG_OPS = (("color", L.DIFFAUG_COLOR), ("translation", L.DIFFAUG_TRANSLATION), ("cutout", L.DIFFAUG_CUTOUT))
+DIFFAUG_OPS = (("color", L.DIFFAUG_COLOR), ("xflip", L.DIFFAUG_XFLIP), ("geometric", L.DIFFAUG_GEOMETRIC),
+               ("translation", L.DIFFAUG_TRANSLATION), ("cutout", L.DIFFAUG_CUTOUT))
+DIFFAUG_GEOM_OPS = L.DIFFAUG_XFLIP | L.DIFFAUG_GEOMETRIC
 
 
 def parse_diff_augment(policy):
-    """'cutout,color' -> ('color', 'cutout'), the bits of the C ABI: the ops always run in DiffAugment's order color ->
-    translation -> cutout, whatever the order of the string.  '' -> ((), 0)."""
+    """'cutout,color' -> ('color', 'cutout'), the bits of the C ABI: the ops always run in the order color -> xflip ->
+    geometric -> translation -> cutout, whatever the order of the string.  '' -> ((), 0)."""
     names = [s.strip() for s in (policy or '').split(',') if s.strip()]
     known = dict(DIFFAUG_OPS)
     bad = [n for n in names if n not in known]
@@ -1365,11 +1367,28 @@ def diffaug_draw_p(state, p, B, index_offset, H, W):
     return rec, mask
 
 
-def _d_input_aug_fwd(ctx, seg, fake, real, cpad, params, policy, opmask):
+def diffaug_draw_geom(state, p, B, index_offset, H, W):
+    """diffaug_draw_p plus the mirror and geometric draws (--diff_augment xflip / geometric): -> the [B, 6] records, bit
+    for bit diffaug_draw's, [B, 8] fp32 inverse matrices M (six entries, two zero pads), and [B] int32 masks whose
+    COLOR / TRANSLATION / CUTOUT bits are diffaug_draw_p's, plus XFLIP (mirror applied) and GEOMETRIC (a geometric gate
+    passed)."""
+    assert state.dtype == torch.int64 and state.numel() == 2 and state.is_contiguous()
+    assert p.dtype == torch.float64 and p.numel() == 1 and p.device == state.device
+    rec = torch.empty(B, L.DIFFAUG_RECORD, dtype=F32, device=state.device)
+    geom = torch.empty(B, L.DIFFAUG_GEOM_RECORD, dtype=F32, device=state.device)
+    mask = torch.empty(B, dtype=torch.int32, device=state.device)
+    L.call("s2e_diffaug_draw_geom", L.ptr(state), L.ptr(p), B, index_offset, H, W, L.ptr(rec), L.ptr(geom), L.ptr(mask),
+           L.stream())
+    return rec, geom, mask
+
+
+def _d_input_aug_fwd(ctx, seg, fake, real, cpad, params, policy, opmask, geom=None):
     seg, fake, real = _c(seg.float()), _c(fake.float()), _c(real.float())
     B, nc, H, W = seg.shape
     assert fake.shape == (B, 1, H, W) and real.shape == (B, 1, H, W), (fake.shape, real.shape, seg.shape)
     assert params.shape == (B, L.DIFFAUG_RECORD) and params.dtype == F32 and params.is_contiguous()
+    if geom is not None and policy & L.DIFFAUG_GEOMETRIC and (H < 2 or W < 2):
+        raise ValueError("--diff_augment geometric needs maps of at least 2 x 2 pixels, got %d x %d" % (H, W))
     cpad = max(cpad, nc + 1)
     st = L.stream()
     means = None
@@ -1377,7 +1396,13 @@ def _d_input_aug_fwd(ctx, seg, fake, real, cpad, params, policy, opmask):
         means = torch.empty(2 * B, dtype=F32, device=seg.device)
         L.call("s2e_diffaug_means", L.ptr(fake), L.ptr(real), B, H, W, L.ptr(means), st)
     out = torch.empty(2 * B, H, W, cpad, dtype=BF16, device=seg.device)
-    if opmask is None:
+    if geom is not None:
+        assert opmask.shape == (B,) and opmask.dtype == torch.int32 and opmask.is_contiguous()
+        assert geom.shape == (B, L.DIFFAUG_GEOM_RECORD) and geom.dtype == F32 and geom.is_contiguous()
+        L.call("s2e_make_d_input_aug_geom", L.ptr(seg), L.ptr(fake), L.ptr(real), B, nc, H, W, cpad, L.ptr(params),
+               L.ptr(means), policy, L.ptr(opmask), L.ptr(geom), L.ptr(out), st)
+        ctx.save_for_backward(params, opmask, geom)
+    elif opmask is None:
         L.call("s2e_make_d_input_aug", L.ptr(seg), L.ptr(fake), L.ptr(real), B, nc, H, W, cpad, L.ptr(params), L.ptr(means),
                policy, L.ptr(out), st)
         ctx.save_for_backward(params)
@@ -1396,12 +1421,16 @@ def _d_input_aug_bwd(ctx, dout):
     dout = _c(dout)
     if not ctx.needs_input_grad[1]:
         return None
-    params, *opmask = ctx.saved_tensors
+    params, *opmask = ctx.saved_tensors       # [], [opmask] or [opmask, geom]
     dfake = torch.empty(B, 1, H, W, dtype=F32, device=dout.device)
     scratch = torch.empty(B, dtype=torch.float64, device=dout.device) if ctx.policy & L.DIFFAUG_COLOR else None
     if not opmask:
         L.call("s2e_d_input_grad_aug", L.ptr(dout), B, nc, H, W, ctx.cpad, L.ptr(params), ctx.policy, L.ptr(scratch),
                L.ptr(dfake), L.stream())
+    elif len(opmask) == 2:
+        mask, geom = opmask
+        L.call("s2e_d_input_grad_aug_geom", L.ptr(dout), B, nc, H, W, ctx.cpad, L.ptr(params), ctx.policy, L.ptr(mask),
+               L.ptr(geom), L.ptr(scratch), L.ptr(dfake), L.stream())
     else:
         L.call("s2e_d_input_grad_aug_masked", L.ptr(dout), B, nc, H, W, ctx.cpad, L.ptr(params), ctx.policy, L.ptr(opmask[0]),
                L.ptr(scratch), L.ptr(dfake), L.stream())
@@ -1432,6 +1461,20 @@ class MakeDInputAugMaskedFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dout):
         return None, _d_input_aug_bwd(ctx, dout), None, None, None, None, None
+
+
+class MakeDInputAugGeomFn(torch.autograd.Function):
+    """MakeDInputAugMaskedFn with the mirror and the geometric warp (--diff_augment xflip / geometric): sample b applies
+    policy & opmask[b] and the matrix geom[b] (ops.diffaug_draw_geom).  The labels are sampled at the nearest tap, the
+    image bilinearly, both with reflection at the borders; the adjoint is a deterministic gather."""
+
+    @staticmethod
+    def forward(ctx, seg, fake, real, cpad, params, opmask, geom, policy):
+        return _d_input_aug_fwd(ctx, seg, fake, real, cpad, params, policy, opmask, geom)
+
+    @staticmethod
+    def backward(ctx, dout):
+        return None, _d_input_aug_bwd(ctx, dout), None, None, None, None, None, None
 
 
 def ada_update(state, target, kimg, interval):
